@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ELBA overlap-detection front end (k-mer count -> A -> A*A^T SpGEMM) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic reads:
   value  reads/s with the packed reads already resident in HBM when the timed region starts
@@ -178,6 +178,49 @@ def run_cpu_reference(dna, k, lo, up, ranks: int):
     return dna.size() / dt, kind, cores, {a: float(b) for a, b in secs.items()}
 
 
+DUMP_SAMPLE = 1 << 18       # entries kept of each large output: at most 2^18 x (3 + 3 + 7) float64 values, 27 MB in all
+DUMP_SIZES = ("nreads", "num_kmers", "distinct", "reliable", "nnzA_pre", "nnzA", "products", "nnzB_pre", "nnzB")
+
+
+def _sample(n: int, m: int) -> np.ndarray:
+    """Sorted indices of a fixed, seeded sample of m out of n entries (all of them when n <= m)."""
+    if n <= m:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+
+
+def dump_outputs(ctx, out_dir: str, sizes: dict, rank: int, world: int, r0: int):
+    """Write what the last resident step (the timed value) returned to its caller as float64 .npy files under out_dir,
+    so that two builds can be compared output for output.  Called on every rank: on several GPUs ctx.kmers() is
+    collective (the super-k-mer path all-gathers the list from its owners).  The files:
+      sizes.npy   the whole-job sizes of DUMP_SIZES
+      kmers.npy   [value >> 32, value & 0xffffffff, count] of the reliable k-mers (float64 is exact below 2^53 only)
+      A.npy       [read, k-mer column, position] of A's entries
+      B.npy       [row read, column read, numshared, s0.q, s0.t, s1.q, s1.t] of B's entries
+    Global read ids; A and B row-major, k-mers ascending.  Large outputs are sampled by _sample, the same entry indices
+    for the same sizes.  On several GPUs every rank writes its own block of A and B (file names end in .rank<r>), and
+    each rank keeps a 1/world share of the sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    m = DUMP_SAMPLE // world
+    tag = "" if world == 1 else f".rank{rank}"
+
+    def save(name, cols):
+        np.save(os.path.join(out_dir, name + ".npy"), np.stack([np.asarray(c, np.float64) for c in cols], axis=1))
+
+    kmers, counts = ctx.kmers()             # the whole list on every rank
+    if rank == 0:
+        np.save(os.path.join(out_dir, "sizes.npy"), np.array([sizes[a] for a in DUMP_SIZES], np.float64))
+        i = _sample(len(kmers), m)
+        save("kmers", (kmers[i] >> np.uint64(32), kmers[i] & np.uint64(0xFFFFFFFF), counts[i]))
+    rp, col, pos = ctx.A()                  # the rows of this rank's reads, global column ids
+    i = _sample(len(col), m)
+    save("A" + tag, (np.searchsorted(rp, i, side="right") - 1 + r0, col[i], pos[i]))
+    rp, col, num, seeds = ctx.B()           # this rank's block of B, local row / column ids
+    info = ctx.comm_info()
+    i = _sample(len(col), m)
+    save("B" + tag, (np.searchsorted(rp, i, side="right") - 1 + info["row0"], col[i].astype(np.int64) + info["col0"], num[i], *seeds[i].T))
+
+
 def square_ranks():
     cores = os.cpu_count() or 1
     q = int(np.floor(np.sqrt(min(cores, 64))))
@@ -194,7 +237,12 @@ def main():
     ap.add_argument("--partitions", type=int, default=0)
     ap.add_argument("--scale", type=float, default=1.0, help="shrink a synthetic workload (debug only; the JSON says so)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed resident steps, write a sample of what the last one computed as .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     w = WORKLOADS[args.workload]
@@ -317,7 +365,9 @@ def main():
     sizes_local = ctx.sizes()
     sizes = ctx.sizes_global()              # whole-job totals (collective)
     digests = ctx.digests()                 # whole-job result digests of the last timed pass (collective)
-    ms_e2e, tm_e2e = timed(step_e2e, max(2, args.steps // 2), 1)
+    if args.dump_outputs:
+        dump_outputs(ctx, args.dump_outputs, sizes, rank, world, r0)
+    ms_e2e, tm_e2e = timed(step_e2e, args.steps, 1)
     sizes_e2e = ctx.sizes()
     digests_e2e = ctx.digests()
     info = ctx.comm_info()
