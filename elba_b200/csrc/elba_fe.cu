@@ -14,6 +14,7 @@
 #include "fasta_ingest.cuh"
 #include "dcsc.cuh"
 #include "transitive.cuh"
+#include "overlap_graph.cuh"
 #include "comm.cuh"
 #include <cub/cub.cuh>
 #include <string>
@@ -108,6 +109,10 @@ struct elba_fe_ctx
     DevBuf tr_in_row, tr_in_col, tr_in_f, tr_key, tr_key2, tr_val, tr_val2, tr_head, tr_okey, tr_row, tr_col, tr_dir, tr_dirT, tr_suf, tr_sufT, tr_src, tr_tr,
            tr_rowptr, tr_I, tr_T, tr_keep, tr_orow, tr_ocol, tr_of, tr_osrc, tr_otr;      // elba_fe_transitive_reduction
     u64 tr_out = 0; bool tr_done = false;
+    // elba_fe_overlap_graph: contained flags, keep scan, this rank's kept alignments (several GPUs), the whole R (job-relative ids)
+    DevBuf og_cont, og_keep, og_lrow, og_lcol, og_lf, og_lsrc, og_row, og_col, og_f, og_src;
+    // og_aligned: the resident alignments are those of the current B (count, build_A and spgemm clear it, align sets it)
+    u64 og_nnz = 0, og_nreads = 0; int64_t og_base = 0; std::vector<u64> og_counts; bool og_aligned = false, og_done = false; cudaEvent_t og_e0 = nullptr, og_e1 = nullptr;
     DevBuf xa_buf, xa_off, xa_len;                          // elba_fe_align on several GPUs: arena and read tables of all ranks
     DevBuf fa_raw, fa_rec, fa_items;                       // elba_fe_ingest_fasta: the raw FASTA chunk, its .fai records, first work item of every read
     DevBuf dc_key, dc_key2, dc_val, dc_val2, dc_head, dc_jc, dc_cp, dc_ir, dc_num, dc_seeds; u64 dc_nzc = 0; bool dc_built = false;      // B by column (DCSC)
@@ -302,6 +307,7 @@ int elba_fe_create(const elba_fe_config *cfg, elba_fe_ctx **out)
     cudaEventCreate(&ctx->up_t0);
     cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming); cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming);
     cudaEventCreate(&ctx->ev_x0); cudaEventCreate(&ctx->ev_x1); cudaEventCreate(&ctx->xd_e0); cudaEventCreate(&ctx->xd_e1);
+    cudaEventCreate(&ctx->og_e0); cudaEventCreate(&ctx->og_e1);
     if (ctx->tmp64.ensure(8192) != cudaSuccess || ctx->ctr.ensure(128) != cudaSuccess) { elba_fe_destroy(ctx); return fail(nullptr, ELBA_FE_ERR_OOM, "cudaMalloc failed"); }
     if (const char *e = getenv("ELBA_FE_TRACE")) ctx->trace = atoi(e) != 0;
     if (const char *e = getenv("ELBA_FE_SCRATCH_MB")) { long v = atol(e); if (v >= 8 && v <= 65536) ctx->scratch_mb = (u64)v; }
@@ -331,6 +337,7 @@ int elba_fe_destroy(elba_fe_ctx *ctx)
         &ctx->tr_in_row, &ctx->tr_in_col, &ctx->tr_in_f, &ctx->tr_key, &ctx->tr_key2, &ctx->tr_val, &ctx->tr_val2, &ctx->tr_head, &ctx->tr_okey, &ctx->tr_row, &ctx->tr_col,
         &ctx->tr_dir, &ctx->tr_dirT, &ctx->tr_suf, &ctx->tr_sufT, &ctx->tr_src, &ctx->tr_tr, &ctx->tr_rowptr, &ctx->tr_I, &ctx->tr_T, &ctx->tr_keep, &ctx->tr_orow, &ctx->tr_ocol,
         &ctx->tr_of, &ctx->tr_osrc, &ctx->tr_otr,
+        &ctx->og_cont, &ctx->og_keep, &ctx->og_lrow, &ctx->og_lcol, &ctx->og_lf, &ctx->og_lsrc, &ctx->og_row, &ctx->og_col, &ctx->og_f, &ctx->og_src,
         &ctx->xa_buf, &ctx->xa_off, &ctx->xa_len, &ctx->fa_raw, &ctx->fa_rec, &ctx->fa_items, &ctx->dc_key, &ctx->dc_key2, &ctx->dc_val, &ctx->dc_val2, &ctx->dc_head, &ctx->dc_jc, &ctx->dc_cp, &ctx->dc_ir, &ctx->dc_num, &ctx->dc_seeds,
         &ctx->plan, &ctx->bfill, &ctx->ovf, &ctx->scratch[0], &ctx->scratch[1], &ctx->skm_slab, &ctx->skm_fill, &ctx->skm_ovf, &ctx->seeds, &ctx->perm, &ctx->rel_idx, &ctx->rel_idx_s,
         &ctx->recvbuf, &ctx->recvcnt, &ctx->tmp64, &ctx->rel_all_key, &ctx->rel_all_cnt, &ctx->g_key, &ctx->g_pos, &ctx->pack_key, &ctx->l_rowptr, &ctx->l_col,
@@ -350,6 +357,8 @@ int elba_fe_destroy(elba_fe_ctx *ctx)
     if (ctx->ev_x1) cudaEventDestroy(ctx->ev_x1);
     if (ctx->xd_e0) cudaEventDestroy(ctx->xd_e0);
     if (ctx->xd_e1) cudaEventDestroy(ctx->xd_e1);
+    if (ctx->og_e0) cudaEventDestroy(ctx->og_e0);
+    if (ctx->og_e1) cudaEventDestroy(ctx->og_e1);
     delete ctx;
     return 0;
 }
@@ -966,6 +975,7 @@ int elba_fe_count(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 1) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_count: no reads uploaded");
+    ctx->og_aligned = ctx->og_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     const int k = ctx->cfg.k, stride = ctx->cfg.stride; const u32 lower = ctx->cfg.lower, upper = ctx->cfg.upper;
     cudaStream_t st = ctx->stream;
@@ -1436,6 +1446,7 @@ int elba_fe_build_A(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 2) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_build_A: call elba_fe_count first");
+    ctx->og_aligned = ctx->og_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     ReadsView rv = view(ctx);
@@ -1624,6 +1635,7 @@ int elba_fe_spgemm(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 3) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_spgemm: call elba_fe_build_A first");
+    ctx->og_aligned = ctx->og_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     const u32 N = ctx->op.l_rows; const u64 nnzA = ctx->op.l_nnz;       // rows of this GPU's block of B
@@ -2074,6 +2086,7 @@ int elba_fe_align(elba_fe_ctx *ctx, int mat, int mis, int gap, int dropoff, uint
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_align: call elba_fe_spgemm first");
     if (mat <= 0 || mis > 0 || gap >= 0 || dropoff < 0) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_align: need mat > 0, mis <= 0, gap < 0, dropoff >= 0");
+    ctx->og_aligned = ctx->og_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     const u64 nnz = ctx->sz.nnzB; const u32 N = ctx->b_rows;
@@ -2150,7 +2163,7 @@ int elba_fe_align(elba_fe_ctx *ctx, int mat, int mis, int gap, int dropoff, uint
     CK(cudaEventRecord(ctx->xd_e1, st));
     CK(cudaStreamSynchronize(st));
     float ms = 0; if (cudaEventElapsedTime(&ms, ctx->xd_e0, ctx->xd_e1) == cudaSuccess) ctx->tm.align_ms = ms;
-    ctx->xd_pairs = np; ctx->xd_done = true;
+    ctx->xd_pairs = np; ctx->xd_done = true; ctx->og_aligned = true;
     if (npairs) *npairs = np;
     return 0;
 }
@@ -2178,34 +2191,19 @@ int elba_fe_get_alignments(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32_t
 }
 
 // ---- transitive reduction of the overlap graph (transitive.cuh): TransitiveReduction(R), src/TransitiveReduction.cpp:3-92 ----
-int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int64_t *col, const int32_t *fields, uint64_t nnz, int64_t nreads,
-                                 int32_t fuzz, uint64_t *nnz_out)
+// The kernel chain on nnz device-resident triples with read ids in [0, n); id_base is added to the string graph's rows and
+// columns.  The caller has recorded ev[0] on the stream; this ends with ev[1], a stream synchronise and tr_done set.
+static int tr_reduce_device(elba_fe_ctx *ctx, const int64_t *row, const int64_t *col, const int32_t *fields, u64 nnz, u32 n, int32_t fuzz,
+                            int64_t id_base, uint64_t *nnz_out)
 {
-    if (!ctx) return ELBA_FE_ERR_INVALID;
-    if (nreads < 0 || nreads >= 0xFFFFFFF0ll) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: bad number of reads");
-    if (nnz >= (1ull << 31)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: more than 2^31 overlaps");
-    if (nnz && (!row || !col || !fields)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: null triples");
-    for (u64 e = 0; e < nnz; ++e)
-    {
-        if (row[e] < 0 || row[e] >= nreads || col[e] < 0 || col[e] >= nreads) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: read id out of range");
-        if (fields[4 * e] < -1 || fields[4 * e] > 3 || fields[4 * e + 1] < -1 || fields[4 * e + 1] > 3)
-            return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: direction outside -1..3 (include/Overlap.hpp:36-44)");
-    }
-    CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
-    ctx->tr_done = false; ctx->tr_out = 0;
-    const u64 m2 = 2 * nnz; const u32 n = (u32)nreads;
+    const u64 m2 = 2 * nnz;
     int rc;
-    CK(cudaEventRecord(ctx->ev[0], st));
     u64 M = 0;
     if (nnz)
     {
-        CK(ctx->tr_in_row.ensure(8 * nnz)); CK(ctx->tr_in_col.ensure(8 * nnz)); CK(ctx->tr_in_f.ensure(16 * nnz));
-        CK(cudaMemcpyAsync(ctx->tr_in_row.p, row, 8 * nnz, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(ctx->tr_in_col.p, col, 8 * nnz, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(ctx->tr_in_f.p, fields, 16 * nnz, cudaMemcpyHostToDevice, st));
         CK(ctx->tr_key.ensure(8 * m2)); CK(ctx->tr_key2.ensure(8 * m2)); CK(ctx->tr_val.ensure(4 * m2)); CK(ctx->tr_val2.ensure(4 * m2)); CK(ctx->tr_head.ensure(8 * (m2 + 1)));
-        k_tr_items<<<nblk(nnz, 256), 256, 0, st>>>(ctx->tr_in_row.as<int64_t>(), ctx->tr_in_col.as<int64_t>(), nnz, ctx->tr_key.as<u64>(), ctx->tr_val.as<u32>()); CKL(); LAUNCHED(ctx);
+        k_tr_items<<<nblk(nnz, 256), 256, 0, st>>>(row, col, nnz, ctx->tr_key.as<u64>(), ctx->tr_val.as<u32>()); CKL(); LAUNCHED(ctx);
         if ((rc = sort_pairs(ctx, ctx->tr_key.as<u64>(), ctx->tr_key2.as<u64>(), ctx->tr_val.as<u32>(), ctx->tr_val2.as<u32>(), m2, 0, 32 + bits_for(std::max<u64>(n, 2))))) return rc;
         k_tr_heads<<<nblk(m2 + 1, 256), 256, 0, st>>>(ctx->tr_key2.as<u64>(), m2, ctx->tr_head.as<u64>()); CKL(); LAUNCHED(ctx);
         if ((rc = exclusive_scan_inplace(ctx, ctx->tr_head.as<u64>(), m2 + 1))) return rc;
@@ -2217,7 +2215,7 @@ int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int
         CK(ctx->tr_okey.ensure(8 * M)); CK(ctx->tr_row.ensure(4 * M)); CK(ctx->tr_col.ensure(4 * M)); CK(ctx->tr_dir.ensure(4 * M)); CK(ctx->tr_dirT.ensure(4 * M));
         CK(ctx->tr_suf.ensure(4 * M)); CK(ctx->tr_sufT.ensure(4 * M)); CK(ctx->tr_src.ensure(4 * M)); CK(ctx->tr_tr.ensure(M)); CK(ctx->tr_rowptr.ensure(8 * ((u64)n + 2)));
         CK(ctx->tr_I.ensure(M)); CK(ctx->tr_T.ensure(M)); CK(ctx->tr_keep.ensure(8 * (M + 1)));
-        k_tr_entries<<<nblk(m2, 256), 256, 0, st>>>(ctx->tr_key2.as<u64>(), ctx->tr_val2.as<u32>(), ctx->tr_head.as<u64>(), m2, nnz, ctx->tr_in_f.as<int32_t>(),
+        k_tr_entries<<<nblk(m2, 256), 256, 0, st>>>(ctx->tr_key2.as<u64>(), ctx->tr_val2.as<u32>(), ctx->tr_head.as<u64>(), m2, nnz, fields,
             ctx->tr_okey.as<u64>(), ctx->tr_row.as<u32>(), ctx->tr_col.as<u32>(), ctx->tr_dir.as<int32_t>(), ctx->tr_dirT.as<int32_t>(), ctx->tr_suf.as<int32_t>(), ctx->tr_sufT.as<int32_t>(),
             ctx->tr_src.as<u32>(), ctx->tr_tr.as<uint8_t>()); CKL(); LAUNCHED(ctx);
         k_segment_ptr<<<nblk((u64)n + 1, 256), 256, 0, st>>>(ctx->tr_okey.as<u64>(), M, n, 32, ctx->tr_rowptr.as<int64_t>()); CKL(); LAUNCHED(ctx);
@@ -2235,6 +2233,11 @@ int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int
         CK(ctx->tr_orow.ensure(8 * S1)); CK(ctx->tr_ocol.ensure(8 * S1)); CK(ctx->tr_of.ensure(16 * S1)); CK(ctx->tr_osrc.ensure(8 * S1)); CK(ctx->tr_otr.ensure(S1));
         k_tr_output<<<nblk(M, 256), 256, 0, st>>>(g, ctx->tr_T.as<uint8_t>(), ctx->tr_keep.as<u64>(), ctx->tr_src.as<u32>(), ctx->tr_tr.as<uint8_t>(),
             ctx->tr_orow.as<int64_t>(), ctx->tr_ocol.as<int64_t>(), ctx->tr_of.as<int32_t>(), ctx->tr_osrc.as<u64>(), ctx->tr_otr.as<uint8_t>()); CKL(); LAUNCHED(ctx);
+        if (id_base && S)
+        {
+            k_add_u64<<<nblk(S, 256), 256, 0, st>>>(ctx->tr_orow.as<u64>(), S, (u64)id_base); CKL(); LAUNCHED(ctx);
+            k_add_u64<<<nblk(S, 256), 256, 0, st>>>(ctx->tr_ocol.as<u64>(), S, (u64)id_base); CKL(); LAUNCHED(ctx);
+        }
         ctx->tr_out = S;
     }
     CK(cudaEventRecord(ctx->ev[1], st));
@@ -2243,6 +2246,133 @@ int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int
     ctx->tr_done = true;
     if (nnz_out) *nnz_out = ctx->tr_out;
     return 0;
+}
+
+int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int64_t *col, const int32_t *fields, uint64_t nnz, int64_t nreads,
+                                 int32_t fuzz, uint64_t *nnz_out)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (nreads < 0 || nreads >= 0xFFFFFFF0ll) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: bad number of reads");
+    if (nnz >= (1ull << 31)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: more than 2^31 overlaps");
+    if (nnz && (!row || !col || !fields)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: null triples");
+    for (u64 e = 0; e < nnz; ++e)
+    {
+        if (row[e] < 0 || row[e] >= nreads || col[e] < 0 || col[e] >= nreads) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: read id out of range");
+        if (fields[4 * e] < -1 || fields[4 * e] > 3 || fields[4 * e + 1] < -1 || fields[4 * e + 1] > 3)
+            return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_transitive_reduction: direction outside -1..3 (include/Overlap.hpp:36-44)");
+    }
+    CK(cudaSetDevice(ctx->cfg.device));
+    cudaStream_t st = ctx->stream;
+    ctx->tr_done = false; ctx->tr_out = 0;
+    CK(cudaEventRecord(ctx->ev[0], st));
+    if (nnz)
+    {
+        CK(ctx->tr_in_row.ensure(8 * nnz)); CK(ctx->tr_in_col.ensure(8 * nnz)); CK(ctx->tr_in_f.ensure(16 * nnz));
+        CK(cudaMemcpyAsync(ctx->tr_in_row.p, row, 8 * nnz, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(ctx->tr_in_col.p, col, 8 * nnz, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(ctx->tr_in_f.p, fields, 16 * nnz, cudaMemcpyHostToDevice, st));
+    }
+    return tr_reduce_device(ctx, ctx->tr_in_row.as<int64_t>(), ctx->tr_in_col.as<int64_t>(), ctx->tr_in_f.as<int32_t>(), nnz, (u32)nreads, fuzz, 0, nnz_out);
+}
+
+// ---- the overlap graph R from the resident alignments (overlap_graph.cuh): the prunes of src/main.cpp:300-313 ------------
+int elba_fe_overlap_graph(elba_fe_ctx *ctx, uint64_t *nnz, uint64_t *ncontained)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->og_aligned || !ctx->xd_done || ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_overlap_graph: call elba_fe_align first");
+    CK(cudaSetDevice(ctx->cfg.device));
+    cudaStream_t st = ctx->stream;
+    ctx->og_done = false;
+    const int W = ctx->comm.nranks;
+    const u64 np = ctx->xd_pairs, Nt = W > 1 ? ctx->N_total : (u64)ctx->n;
+    // job-relative id of this block's first row / column read (one GPU: 0)
+    const u32 row_base = (u32)(ctx->op.row0 - ctx->read_base0), col_base = (u32)(ctx->op.col0 - ctx->read_base0);
+    const u32 *prow = ctx->xd_prow.as<u32>(), *pcol = ctx->xd_pcol.as<u32>(); const int32_t *fields = ctx->xd_out.as<int32_t>();
+    int rc;
+    CK(cudaEventRecord(ctx->og_e0, st));
+    // C over the alignments of every rank: local flags, then one max-all-reduce of the bytes
+    CK(ctx->og_cont.ensure(std::max<u64>(Nt, 1))); CK(ctx->og_keep.ensure(8 * (np + 2)));      // np + 1 keep flags, |C| behind them
+    if (Nt) CK(cudaMemsetAsync(ctx->og_cont.p, 0, Nt, st));
+    if (np) { k_og_contained<<<nblk(np, 256), 256, 0, st>>>(prow, pcol, fields, np, row_base, col_base, ctx->og_cont.as<uint8_t>()); CKL(); LAUNCHED(ctx); }
+    if (W > 1 && Nt) NC(ctx->comm.api->AllReduce(ctx->og_cont.p, ctx->og_cont.p, (size_t)Nt, ncclUint8, ncclMax, ctx->comm.comm, st));
+    u64 *d_ncont = ctx->og_keep.as<u64>() + np + 1;
+    CK(cudaMemsetAsync(d_ncont, 0, 8, st));
+    if (Nt) { k_og_count<<<(u32)std::min<u64>(nblk(Nt, 256), (u64)grid_for(ctx, 4)), 256, 0, st>>>(ctx->og_cont.as<uint8_t>(), Nt, d_ncont); CKL(); LAUNCHED(ctx); }
+    // keep flags -> positions -> this rank's part of R
+    k_og_keep<<<nblk(np + 1, 256), 256, 0, st>>>(prow, pcol, fields, np, row_base, col_base, ctx->og_cont.as<uint8_t>(), ctx->og_keep.as<u64>()); CKL(); LAUNCHED(ctx);
+    if ((rc = exclusive_scan_inplace(ctx, ctx->og_keep.as<u64>(), np + 1))) return rc;
+    u64 h[2] = {0, 0};
+    CK(cudaMemcpyAsync(&h[0], ctx->og_keep.as<u64>() + np, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&h[1], d_ncont, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const u64 kept = h[0];
+    DevBuf *dst[4] = { &ctx->og_row, &ctx->og_col, &ctx->og_f, &ctx->og_src };
+    if (W > 1) { dst[0] = &ctx->og_lrow; dst[1] = &ctx->og_lcol; dst[2] = &ctx->og_lf; dst[3] = &ctx->og_lsrc; }
+    const u64 k1 = std::max<u64>(kept, 1);
+    CK(dst[0]->ensure(8 * k1)); CK(dst[1]->ensure(8 * k1)); CK(dst[2]->ensure(16 * k1)); CK(dst[3]->ensure(8 * k1));
+    if (kept)
+    {
+        k_og_compact<<<nblk(np, 256), 256, 0, st>>>(prow, pcol, fields, np, row_base, col_base, ctx->og_keep.as<u64>(),
+            dst[0]->as<int64_t>(), dst[1]->as<int64_t>(), dst[2]->as<int32_t>(), dst[3]->as<u64>()); CKL(); LAUNCHED(ctx);
+    }
+    // several GPUs: every rank gets the whole R, the ranks' parts in rank order
+    u64 total = kept;
+    if ((rc = allgather_u64(ctx, kept, ctx->og_counts))) return rc;
+    if (W > 1)
+    {
+        total = 0; for (u64 c : ctx->og_counts) total += c;
+        const u64 t1 = std::max<u64>(total, 1);
+        CK(ctx->og_row.ensure(8 * t1)); CK(ctx->og_col.ensure(8 * t1)); CK(ctx->og_f.ensure(16 * t1)); CK(ctx->og_src.ensure(8 * t1));
+        if ((rc = allgatherv(ctx, ctx->og_lrow.p, ctx->og_row.p, ctx->og_counts, 8))) return rc;
+        if ((rc = allgatherv(ctx, ctx->og_lcol.p, ctx->og_col.p, ctx->og_counts, 8))) return rc;
+        if ((rc = allgatherv(ctx, ctx->og_lf.p, ctx->og_f.p, ctx->og_counts, 16))) return rc;
+        if ((rc = allgatherv(ctx, ctx->og_lsrc.p, ctx->og_src.p, ctx->og_counts, 8))) return rc;
+    }
+    CK(cudaEventRecord(ctx->og_e1, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0; if (cudaEventElapsedTime(&ms, ctx->og_e0, ctx->og_e1) == cudaSuccess) ctx->tm.overlap_ms = ms;
+    ctx->og_nnz = total; ctx->og_nreads = Nt; ctx->og_base = ctx->read_base0; ctx->og_done = true;
+    if (nnz) *nnz = total;
+    if (ncontained) *ncontained = h[1];
+    return 0;
+}
+
+int elba_fe_get_overlap_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32_t *fields, int32_t *src_rank, uint64_t *src_pair)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->og_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_get_overlap_graph: call elba_fe_overlap_graph first");
+    CK(cudaSetDevice(ctx->cfg.device));
+    const u64 m = ctx->og_nnz;
+    if (!m) return 0;
+    DevBuf tmp;
+    if (row || col)
+    {
+        CK(tmp.ensure(16 * m));
+        k_og_ids<<<nblk(m, 256), 256, 0, ctx->stream>>>(ctx->og_row.as<int64_t>(), ctx->og_col.as<int64_t>(), m, ctx->og_base, tmp.as<int64_t>(), tmp.as<int64_t>() + m);
+        LAUNCHED(ctx);
+    }
+    D2H(row, tmp.p, 8 * m); D2H(col, tmp.as<int64_t>() + m, 8 * m); D2H(fields, ctx->og_f.p, 16 * m); D2H(src_pair, ctx->og_src.p, 8 * m);
+    if (src_rank)
+    {
+        u64 o = 0;
+        for (size_t r = 0; r < ctx->og_counts.size(); ++r) for (u64 i = 0; i < ctx->og_counts[r]; ++i) src_rank[o++] = (int32_t)r;
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    tmp.release();
+    return 0;
+}
+
+int elba_fe_reduce_overlap_graph(elba_fe_ctx *ctx, int32_t fuzz, uint64_t *nnz_out)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->og_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_reduce_overlap_graph: call elba_fe_overlap_graph first");
+    const u64 nnz = ctx->og_nnz, Nt = ctx->og_nreads;
+    if (Nt >= 0xFFFFFFF0ull) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_reduce_overlap_graph: too many reads");
+    if (nnz >= (1ull << 31)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_reduce_overlap_graph: more than 2^31 overlaps");
+    CK(cudaSetDevice(ctx->cfg.device));
+    ctx->tr_done = false; ctx->tr_out = 0;
+    CK(cudaEventRecord(ctx->ev[0], ctx->stream));
+    return tr_reduce_device(ctx, ctx->og_row.as<int64_t>(), ctx->og_col.as<int64_t>(), ctx->og_f.as<int32_t>(), nnz, (u32)Nt, fuzz, ctx->og_base, nnz_out);
 }
 
 int elba_fe_get_string_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32_t *fields, uint64_t *src, uint8_t *transposed)

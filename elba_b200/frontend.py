@@ -49,10 +49,10 @@ class Timings(C.Structure):
     _fields_ = [("upload_ms", C.c_float), ("count_ms", C.c_float), ("build_ms", C.c_float), ("spgemm_ms", C.c_float),
                 ("download_ms", C.c_float), ("count_kernel_ms", C.c_float), ("spgemm_kernel_ms", C.c_float),
                 ("kernel_launches", C.c_uint32), ("partition_ms", C.c_float), ("lookup_ms", C.c_float), ("exchange_ms", C.c_float),
-                ("exchange_mbytes", C.c_float), ("panel_mbytes", C.c_float), ("align_ms", C.c_float), ("transitive_ms", C.c_float), ("reserved", C.c_float * 1)]
+                ("exchange_mbytes", C.c_float), ("panel_mbytes", C.c_float), ("align_ms", C.c_float), ("transitive_ms", C.c_float), ("overlap_ms", C.c_float)]
 
     def as_dict(self):
-        return {n: (int(getattr(self, n)) if n == "kernel_launches" else float(getattr(self, n))) for n, _ in self._fields_ if n != "reserved"}
+        return {n: (int(getattr(self, n)) if n == "kernel_launches" else float(getattr(self, n))) for n, _ in self._fields_}
 
 
 # every symbol include/elba_fe.h declares (tests check the library exports all of them)
@@ -65,6 +65,7 @@ ABI_SYMBOLS = (
     "elba_fe_comm_get_id", "elba_fe_comm_init", "elba_fe_comm_set_grid", "elba_fe_comm_info", "elba_fe_block_extent", "elba_fe_sizes_global",
     "elba_fe_digests", "elba_fe_device_count",
     "elba_fe_transitive_reduction", "elba_fe_get_string_graph",
+    "elba_fe_overlap_graph", "elba_fe_get_overlap_graph", "elba_fe_reduce_overlap_graph",
     "elba_fe_ingest_fasta", "elba_fe_reads_size", "elba_fe_get_reads", "elba_fe_B_dcsc", "elba_fe_get_B_dcsc", "elba_fe_device_B_dcsc",
 )
 
@@ -300,6 +301,29 @@ class Context:
         n = C.c_uint64()
         self._ck(self.L.elba_fe_transitive_reduction(self.h, _p(rows) if len(rows) else None, _p(cols) if len(rows) else None, _p(fields) if len(rows) else None,
                                                      C.c_uint64(len(rows)), C.c_int64(nreads), C.c_int32(fuzz), C.byref(n)))
+        m = n.value
+        orow, ocol, of = np.zeros(m, np.int64), np.zeros(m, np.int64), np.zeros((m, 4), np.int32)
+        osrc, otr = np.zeros(m, np.uint64), np.zeros(m, np.uint8)
+        self._ck(self.L.elba_fe_get_string_graph(self.h, _p(orow), _p(ocol), _p(of), _p(osrc), _p(otr)))
+        return orow, ocol, of, osrc, otr
+
+    def overlap_graph(self):
+        """The overlap graph R from the resident alignments (the prunes of src/main.cpp:300-313, elba_fe_overlap_graph; collective
+        on several GPUs, where every rank gets the whole R): (rows, cols, fields[nnz, 4] = direction, directionT, suffix, suffixT,
+        src_rank, src_pair, ncontained) with global read ids; src_rank / src_pair name the alignment of `align()` on that rank."""
+        n, nc = C.c_uint64(), C.c_uint64()
+        self._ck(self.L.elba_fe_overlap_graph(self.h, C.byref(n), C.byref(nc)))
+        m = n.value
+        rows, cols, f = np.zeros(m, np.int64), np.zeros(m, np.int64), np.zeros((m, 4), np.int32)
+        src_rank, src_pair = np.zeros(m, np.int32), np.zeros(m, np.uint64)
+        self._ck(self.L.elba_fe_get_overlap_graph(self.h, _p(rows), _p(cols), _p(f), _p(src_rank), _p(src_pair)))
+        return rows, cols, f, src_rank, src_pair, int(nc.value)
+
+    def string_graph(self, fuzz: int = 1000):
+        """TransitiveReduction of the resident R (elba_fe_reduce_overlap_graph; call overlap_graph first): the same
+        (rows, cols, fields[nnzS, 4], src, transposed) as transitive_reduction, src indexing R."""
+        n = C.c_uint64()
+        self._ck(self.L.elba_fe_reduce_overlap_graph(self.h, C.c_int32(fuzz), C.byref(n)))
         m = n.value
         orow, ocol, of = np.zeros(m, np.int64), np.zeros(m, np.int64), np.zeros((m, 4), np.int32)
         osrc, otr = np.zeros(m, np.uint64), np.zeros(m, np.uint8)

@@ -232,6 +232,26 @@ int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int
                                  int64_t nreads, int32_t fuzz, uint64_t *nnz_out);
 int elba_fe_get_string_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32_t *fields /* nnz_out x 4 */, uint64_t *src, uint8_t *transposed);
 
+/* ---- from the alignments to the string graph without leaving the device ---------------------------------------------
+ * The prunes between PairwiseAlignment and TransitiveReduction (src/main.cpp:300-313) on the alignments elba_fe_align left
+ * resident, restated in tests/tr_inputs.py::overlap_graph: over the alignments of ALL ranks, C = the rows of the passed
+ * alignments with containedQ and the columns of those with containedT; an alignment stays in the overlap graph R iff it
+ * passed and neither of its reads is in C.  An entry of R is (global row, global column, direction, directionT, suffix,
+ * suffixT); R is the ranks' kept alignments concatenated in rank order, each rank's in the order of elba_fe_get_alignments.
+ * overlap_graph: after elba_fe_align; COLLECTIVE on several GPUs (one all-reduce of one byte per read, then all-gathers):
+ * every rank ends up holding the whole R.  *nnz = entries of R, *ncontained = reads in C.  Only scalars reach the host.
+ * get_overlap_graph: R to the host; any pointer may be NULL; src_rank / src_pair = which rank's alignment the entry is
+ * (the index into that rank's elba_fe_get_alignments order).
+ * reduce_overlap_graph: TransitiveReduction of the resident R, the kernels and semantics of elba_fe_transitive_reduction with
+ * nreads = the reads of the whole job; no collective (every rank reduces its replica).  The result is read with
+ * elba_fe_get_string_graph, where src indexes R.  More than 2^31 entries in R is ELBA_FE_ERR_INVALID.
+ * elba_fe_count, elba_fe_build_A, elba_fe_spgemm and elba_fe_align discard R: the calls after them are ELBA_FE_ERR_STATE
+ * until the next elba_fe_overlap_graph. */
+int elba_fe_overlap_graph(elba_fe_ctx *ctx, uint64_t *nnz, uint64_t *ncontained);
+int elba_fe_get_overlap_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32_t *fields /* nnz x 4 */,
+                              int32_t *src_rank, uint64_t *src_pair);
+int elba_fe_reduce_overlap_graph(elba_fe_ctx *ctx, int32_t fuzz, uint64_t *nnz_out);
+
 /* ---- the reference's sizing sketches, bit-exact (not needed for the result when lower >= 2) ----------- */
 /* HyperLogLog over the canonical k-mers of the uploaded reads exactly as KmerEstimateHandler drives it
  * (include/KmerOps.hpp:58-69, src/HyperLogLog.cpp:40-76): registers[4096] and estimate(). */
@@ -259,8 +279,8 @@ typedef struct {
     float exchange_mbytes;  /* MB this rank sent in it */
     float panel_mbytes;     /* MB this rank received as routed seed triples and in the all-gather of A's row blocks */
     float align_ms;         /* elba_fe_align: pair selection + the X-drop kernel */
-    float transitive_ms;    /* elba_fe_transitive_reduction */
-    float reserved[1];
+    float transitive_ms;    /* elba_fe_transitive_reduction, elba_fe_reduce_overlap_graph */
+    float overlap_ms;       /* elba_fe_overlap_graph (several GPUs: with its all-reduce and all-gathers) */
 } elba_fe_timings_t;
 int elba_fe_timings(elba_fe_ctx *ctx, elba_fe_timings_t *out);
 int elba_fe_reset_timings(elba_fe_ctx *ctx);
