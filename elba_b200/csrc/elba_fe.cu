@@ -15,6 +15,7 @@
 #include "dcsc.cuh"
 #include "transitive.cuh"
 #include "overlap_graph.cuh"
+#include "contigs.cuh"
 #include "comm.cuh"
 #include <cub/cub.cuh>
 #include <string>
@@ -109,11 +110,17 @@ struct elba_fe_ctx
     DevBuf tr_in_row, tr_in_col, tr_in_f, tr_key, tr_key2, tr_val, tr_val2, tr_head, tr_okey, tr_row, tr_col, tr_dir, tr_dirT, tr_suf, tr_sufT, tr_src, tr_tr,
            tr_rowptr, tr_I, tr_T, tr_keep, tr_orow, tr_ocol, tr_of, tr_osrc, tr_otr;      // elba_fe_transitive_reduction
     u64 tr_out = 0; bool tr_done = false;
+    bool tr_resident = false;                               // the tr_* output is the reduction of the current resident R (not of a host R)
     // elba_fe_overlap_graph: contained flags, keep scan, this rank's kept alignments (several GPUs), the whole R (job-relative ids)
     DevBuf og_cont, og_keep, og_lrow, og_lcol, og_lf, og_lsrc, og_row, og_col, og_f, og_src;
     // og_aligned: the resident alignments are those of the current B (count, build_A and spgemm clear it, align sets it)
     u64 og_nnz = 0, og_nreads = 0; int64_t og_base = 0; std::vector<u64> og_counts; bool og_aligned = false, og_done = false; cudaEvent_t og_e0 = nullptr, og_e1 = nullptr;
     DevBuf xa_buf, xa_off, xa_len;                          // elba_fe_align on several GPUs: arena and read tables of all ranks
+    u64 read_gen = 0, xd_read_gen = 0;                      // bumped by every upload / set / ingest of reads; its value at elba_fe_align
+    // elba_fe_contigs: S uploaded by contigs_from_graph, per-read scratch, the layout, this rank's sequences
+    DevBuf ct_in_row, ct_in_col, ct_in_f, ct_ptr, ct_branch, ct_slot, ct_succ[2], ct_dist[2], ct_mn[2], ct_cyc, ct_flag, ct_start, ct_pos, ct_next, ct_L,
+           ct_cptr, ct_read, ct_rev, ct_beg, ct_end, ct_boff, ct_blen, ct_bbyte, ct_packed;
+    elba_fe_contig_info_t ct_info; bool ct_done = false; cudaEvent_t ct_e0 = nullptr, ct_e1 = nullptr;
     DevBuf fa_raw, fa_rec, fa_items;                       // elba_fe_ingest_fasta: the raw FASTA chunk, its .fai records, first work item of every read
     DevBuf dc_key, dc_key2, dc_val, dc_val2, dc_head, dc_jc, dc_cp, dc_ir, dc_num, dc_seeds; u64 dc_nzc = 0; bool dc_built = false;      // B by column (DCSC)
     // multi-GPU
@@ -307,7 +314,7 @@ int elba_fe_create(const elba_fe_config *cfg, elba_fe_ctx **out)
     cudaEventCreate(&ctx->up_t0);
     cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming); cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming);
     cudaEventCreate(&ctx->ev_x0); cudaEventCreate(&ctx->ev_x1); cudaEventCreate(&ctx->xd_e0); cudaEventCreate(&ctx->xd_e1);
-    cudaEventCreate(&ctx->og_e0); cudaEventCreate(&ctx->og_e1);
+    cudaEventCreate(&ctx->og_e0); cudaEventCreate(&ctx->og_e1); cudaEventCreate(&ctx->ct_e0); cudaEventCreate(&ctx->ct_e1);
     if (ctx->tmp64.ensure(8192) != cudaSuccess || ctx->ctr.ensure(128) != cudaSuccess) { elba_fe_destroy(ctx); return fail(nullptr, ELBA_FE_ERR_OOM, "cudaMalloc failed"); }
     if (const char *e = getenv("ELBA_FE_TRACE")) ctx->trace = atoi(e) != 0;
     if (const char *e = getenv("ELBA_FE_SCRATCH_MB")) { long v = atol(e); if (v >= 8 && v <= 65536) ctx->scratch_mb = (u64)v; }
@@ -338,7 +345,10 @@ int elba_fe_destroy(elba_fe_ctx *ctx)
         &ctx->tr_dir, &ctx->tr_dirT, &ctx->tr_suf, &ctx->tr_sufT, &ctx->tr_src, &ctx->tr_tr, &ctx->tr_rowptr, &ctx->tr_I, &ctx->tr_T, &ctx->tr_keep, &ctx->tr_orow, &ctx->tr_ocol,
         &ctx->tr_of, &ctx->tr_osrc, &ctx->tr_otr,
         &ctx->og_cont, &ctx->og_keep, &ctx->og_lrow, &ctx->og_lcol, &ctx->og_lf, &ctx->og_lsrc, &ctx->og_row, &ctx->og_col, &ctx->og_f, &ctx->og_src,
-        &ctx->xa_buf, &ctx->xa_off, &ctx->xa_len, &ctx->fa_raw, &ctx->fa_rec, &ctx->fa_items, &ctx->dc_key, &ctx->dc_key2, &ctx->dc_val, &ctx->dc_val2, &ctx->dc_head, &ctx->dc_jc, &ctx->dc_cp, &ctx->dc_ir, &ctx->dc_num, &ctx->dc_seeds,
+        &ctx->xa_buf, &ctx->xa_off, &ctx->xa_len,
+        &ctx->ct_in_row, &ctx->ct_in_col, &ctx->ct_in_f, &ctx->ct_ptr, &ctx->ct_branch, &ctx->ct_slot, &ctx->ct_succ[0], &ctx->ct_succ[1], &ctx->ct_dist[0], &ctx->ct_dist[1],
+        &ctx->ct_mn[0], &ctx->ct_mn[1], &ctx->ct_cyc, &ctx->ct_flag, &ctx->ct_start, &ctx->ct_pos, &ctx->ct_next, &ctx->ct_L, &ctx->ct_cptr, &ctx->ct_read, &ctx->ct_rev,
+        &ctx->ct_beg, &ctx->ct_end, &ctx->ct_boff, &ctx->ct_blen, &ctx->ct_bbyte, &ctx->ct_packed, &ctx->fa_raw, &ctx->fa_rec, &ctx->fa_items, &ctx->dc_key, &ctx->dc_key2, &ctx->dc_val, &ctx->dc_val2, &ctx->dc_head, &ctx->dc_jc, &ctx->dc_cp, &ctx->dc_ir, &ctx->dc_num, &ctx->dc_seeds,
         &ctx->plan, &ctx->bfill, &ctx->ovf, &ctx->scratch[0], &ctx->scratch[1], &ctx->skm_slab, &ctx->skm_fill, &ctx->skm_ovf, &ctx->seeds, &ctx->perm, &ctx->rel_idx, &ctx->rel_idx_s,
         &ctx->recvbuf, &ctx->recvcnt, &ctx->tmp64, &ctx->rel_all_key, &ctx->rel_all_cnt, &ctx->g_key, &ctx->g_pos, &ctx->pack_key, &ctx->l_rowptr, &ctx->l_col,
         &ctx->r_key, &ctx->r_key2, &ctx->r_pos, &ctx->r_colptr, &ctx->r_row, &ctx->r_ptr };
@@ -359,6 +369,8 @@ int elba_fe_destroy(elba_fe_ctx *ctx)
     if (ctx->xd_e1) cudaEventDestroy(ctx->xd_e1);
     if (ctx->og_e0) cudaEventDestroy(ctx->og_e0);
     if (ctx->og_e1) cudaEventDestroy(ctx->og_e1);
+    if (ctx->ct_e0) cudaEventDestroy(ctx->ct_e0);
+    if (ctx->ct_e1) cudaEventDestroy(ctx->ct_e1);
     delete ctx;
     return 0;
 }
@@ -389,7 +401,7 @@ static int stage_reads(elba_fe_ctx *ctx, const uint8_t *packed, uint64_t packed_
     if (nreads && (!byte_off || !len)) return fail(ctx, ELBA_FE_ERR_INVALID, "null read tables");
     if (packed_bytes && !packed) return fail(ctx, ELBA_FE_ERR_INVALID, "null arena");
     CK(cudaSetDevice(ctx->cfg.device));
-    ctx->phase = 0;
+    ctx->phase = 0; ++ctx->read_gen; ctx->ct_done = false;
     ctx->n = (u32)nreads; ctx->packed_bytes = packed_bytes; ctx->read_id_offset = read_id_offset;
     cudaStream_t st = ctx->stream;
     CK(cudaEventRecord(ctx->ev[0], st));
@@ -491,7 +503,7 @@ int elba_fe_ingest_fasta(elba_fe_ctx *ctx, const char *chunk, uint64_t chunk_byt
         head += nb; nitems += (nb + FI_ITEM_BYTES - 1) / FI_ITEM_BYTES;
     }
     off[nreads] = head; items[nreads] = nitems;
-    ctx->phase = 0;
+    ctx->phase = 0; ++ctx->read_gen; ctx->ct_done = false;
     ctx->n = (u32)nreads; ctx->packed_bytes = head; ctx->read_id_offset = read_id_offset; ctx->up_n = 0;
     cudaStream_t st = ctx->stream;
     CK(cudaEventRecord(ctx->ev[0], st));
@@ -975,7 +987,7 @@ int elba_fe_count(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 1) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_count: no reads uploaded");
-    ctx->og_aligned = ctx->og_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     const int k = ctx->cfg.k, stride = ctx->cfg.stride; const u32 lower = ctx->cfg.lower, upper = ctx->cfg.upper;
     cudaStream_t st = ctx->stream;
@@ -1446,7 +1458,7 @@ int elba_fe_build_A(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 2) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_build_A: call elba_fe_count first");
-    ctx->og_aligned = ctx->og_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     ReadsView rv = view(ctx);
@@ -1635,7 +1647,7 @@ int elba_fe_spgemm(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 3) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_spgemm: call elba_fe_build_A first");
-    ctx->og_aligned = ctx->og_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     const u32 N = ctx->op.l_rows; const u64 nnzA = ctx->op.l_nnz;       // rows of this GPU's block of B
@@ -2086,7 +2098,7 @@ int elba_fe_align(elba_fe_ctx *ctx, int mat, int mis, int gap, int dropoff, uint
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_align: call elba_fe_spgemm first");
     if (mat <= 0 || mis > 0 || gap >= 0 || dropoff < 0) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_align: need mat > 0, mis <= 0, gap < 0, dropoff >= 0");
-    ctx->og_aligned = ctx->og_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     const u64 nnz = ctx->sz.nnzB; const u32 N = ctx->b_rows;
@@ -2163,7 +2175,7 @@ int elba_fe_align(elba_fe_ctx *ctx, int mat, int mis, int gap, int dropoff, uint
     CK(cudaEventRecord(ctx->xd_e1, st));
     CK(cudaStreamSynchronize(st));
     float ms = 0; if (cudaEventElapsedTime(&ms, ctx->xd_e0, ctx->xd_e1) == cudaSuccess) ctx->tm.align_ms = ms;
-    ctx->xd_pairs = np; ctx->xd_done = true; ctx->og_aligned = true;
+    ctx->xd_pairs = np; ctx->xd_done = true; ctx->og_aligned = true; ctx->xd_read_gen = ctx->read_gen;
     if (npairs) *npairs = np;
     return 0;
 }
@@ -2263,7 +2275,7 @@ int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int
     }
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
-    ctx->tr_done = false; ctx->tr_out = 0;
+    ctx->tr_done = ctx->tr_resident = ctx->ct_done = false; ctx->tr_out = 0;
     CK(cudaEventRecord(ctx->ev[0], st));
     if (nnz)
     {
@@ -2282,7 +2294,7 @@ int elba_fe_overlap_graph(elba_fe_ctx *ctx, uint64_t *nnz, uint64_t *ncontained)
     if (!ctx->og_aligned || !ctx->xd_done || ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_overlap_graph: call elba_fe_align first");
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
-    ctx->og_done = false;
+    ctx->og_done = ctx->tr_resident = ctx->ct_done = false;
     const int W = ctx->comm.nranks;
     const u64 np = ctx->xd_pairs, Nt = W > 1 ? ctx->N_total : (u64)ctx->n;
     // job-relative id of this block's first row / column read (one GPU: 0)
@@ -2370,9 +2382,11 @@ int elba_fe_reduce_overlap_graph(elba_fe_ctx *ctx, int32_t fuzz, uint64_t *nnz_o
     if (Nt >= 0xFFFFFFF0ull) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_reduce_overlap_graph: too many reads");
     if (nnz >= (1ull << 31)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_reduce_overlap_graph: more than 2^31 overlaps");
     CK(cudaSetDevice(ctx->cfg.device));
-    ctx->tr_done = false; ctx->tr_out = 0;
+    ctx->tr_done = ctx->ct_done = false; ctx->tr_out = 0;
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
-    return tr_reduce_device(ctx, ctx->og_row.as<int64_t>(), ctx->og_col.as<int64_t>(), ctx->og_f.as<int32_t>(), nnz, (u32)Nt, fuzz, ctx->og_base, nnz_out);
+    const int rc = tr_reduce_device(ctx, ctx->og_row.as<int64_t>(), ctx->og_col.as<int64_t>(), ctx->og_f.as<int32_t>(), nnz, (u32)Nt, fuzz, ctx->og_base, nnz_out);
+    if (rc == 0) ctx->tr_resident = true;
+    return rc;
 }
 
 int elba_fe_get_string_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32_t *fields, uint64_t *src, uint8_t *transposed)
@@ -2382,6 +2396,199 @@ int elba_fe_get_string_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int32
     const u64 S = ctx->tr_out;
     D2H(row, ctx->tr_orow.p, 8 * S); D2H(col, ctx->tr_ocol.p, 8 * S); D2H(fields, ctx->tr_of.p, 16 * S); D2H(src, ctx->tr_osrc.p, 8 * S); D2H(transposed, ctx->tr_otr.p, S);
     CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+// ---- contigs from the string graph (contigs.cuh): the stage GenerateContigs runs in the reference (src/main.cpp:320) ------
+// S: m entries row-major with global ids, base = global id of read 0 of the job, n reads in rd (job-relative ids).  Builds the
+// whole layout on every rank (no collective) and the sequences of the contigs [block of rank / nranks].
+static int contigs_device(elba_fe_ctx *ctx, const int64_t *row, const int64_t *col, const int32_t *f, u64 m, u32 n, int64_t base,
+                          CtReads rd, int rank, int nranks, elba_fe_contig_info_t *info)
+{
+    cudaStream_t st = ctx->stream;
+    int rc;
+    const u64 n1 = (u64)n + 1, ns = 2ull * n;
+    CK(cudaEventRecord(ctx->ct_e0, st));
+    CK(ctx->ct_ptr.ensure(8 * n1)); CK(ctx->ct_branch.ensure(n1)); CK(ctx->ct_slot.ensure(4 * (ns + 2))); CK(ctx->ct_cyc.ensure(n1));
+    for (int i = 0; i < 2; ++i) { CK(ctx->ct_succ[i].ensure(4 * (ns + 2))); CK(ctx->ct_dist[i].ensure(4 * (ns + 2))); CK(ctx->ct_mn[i].ensure(4 * (ns + 2))); }
+    CK(ctx->ct_flag.ensure(8 * n1)); CK(ctx->ct_start.ensure(4 * n1)); CK(ctx->ct_pos.ensure(4 * n1)); CK(ctx->ct_next.ensure(n1)); CK(ctx->ct_L.ensure(4 * n1));
+    CK(ctx->ct_cptr.ensure(8 * n1)); CK(ctx->ct_read.ensure(8 * n1)); CK(ctx->ct_rev.ensure(n1)); CK(ctx->ct_beg.ensure(4 * n1)); CK(ctx->ct_end.ensure(4 * n1));
+    CK(ctx->ct_boff.ensure(8 * n1)); CK(ctx->tmp64.ensure(64));
+    u64 *d_cnt = ctx->tmp64.as<u64>();                    // [0] branches, [1] cycles
+    CK(cudaMemsetAsync(d_cnt, 0, 16, st));
+    CK(cudaMemsetAsync(ctx->ct_cptr.p, 0, 8 * n1, st)); CK(cudaMemsetAsync(ctx->ct_boff.p, 0, 8 * n1, st));
+    if (n)
+    {
+        const u32 gn = nblk(n, 256), gs = nblk(ns, 256);
+        u32 *slot = ctx->ct_slot.as<u32>();
+        k_ct_rowptr<<<nblk(n1, 256), 256, 0, st>>>(row, m, n, base, ctx->ct_ptr.as<u64>()); CKL(); LAUNCHED(ctx);
+        k_ct_branch<<<gn, 256, 0, st>>>(ctx->ct_ptr.as<u64>(), f, n, ctx->ct_branch.as<uint8_t>()); CKL(); LAUNCHED(ctx);
+        k_ct_slots<<<gn, 256, 0, st>>>(ctx->ct_ptr.as<u64>(), col, f, n, base, ctx->ct_branch.as<uint8_t>(), slot); CKL(); LAUNCHED(ctx);
+        // list ranking: rounds doubles the hops every state has looked ahead; 2^rounds >= n covers the longest chain
+        const int rounds = bits_for(std::max<u64>(n, 2));
+        int cur = 0;
+        k_ct_init<<<gs, 256, 0, st>>>(slot, col, n, base, ctx->ct_succ[0].as<u32>(), nullptr, ctx->ct_mn[0].as<u32>()); CKL(); LAUNCHED(ctx);
+        for (int r = 0; r < rounds; ++r, cur ^= 1)
+        {
+            k_ct_jump<<<gs, 256, 0, st>>>(ns, ctx->ct_succ[cur].as<u32>(), nullptr, ctx->ct_mn[cur].as<u32>(), ctx->ct_succ[cur ^ 1].as<u32>(), nullptr, ctx->ct_mn[cur ^ 1].as<u32>());
+            CKL(); LAUNCHED(ctx);
+        }
+        k_ct_cut<<<gn, 256, 0, st>>>(slot, col, base, ctx->ct_succ[cur].as<u32>(), ctx->ct_mn[cur].as<u32>(), n, ctx->ct_cyc.as<uint8_t>()); CKL(); LAUNCHED(ctx);
+        cur = 0;
+        k_ct_init<<<gs, 256, 0, st>>>(slot, col, n, base, ctx->ct_succ[0].as<u32>(), ctx->ct_dist[0].as<u32>(), nullptr); CKL(); LAUNCHED(ctx);
+        for (int r = 0; r < rounds; ++r, cur ^= 1)
+        {
+            k_ct_jump<<<gs, 256, 0, st>>>(ns, ctx->ct_succ[cur].as<u32>(), ctx->ct_dist[cur].as<u32>(), nullptr, ctx->ct_succ[cur ^ 1].as<u32>(), ctx->ct_dist[cur ^ 1].as<u32>(), nullptr);
+            CKL(); LAUNCHED(ctx);
+        }
+        k_ct_place<<<nblk(n1, 256), 256, 0, st>>>(ctx->ct_succ[cur].as<u32>(), ctx->ct_dist[cur].as<u32>(), n, ctx->ct_flag.as<u64>(), ctx->ct_start.as<u32>(),
+            ctx->ct_pos.as<u32>(), ctx->ct_next.as<uint8_t>(), ctx->ct_L.as<u32>()); CKL(); LAUNCHED(ctx);
+        if ((rc = exclusive_scan_inplace(ctx, ctx->ct_flag.as<u64>(), n1))) return rc;
+        k_ct_clen<<<gn, 256, 0, st>>>(ctx->ct_flag.as<u64>(), ctx->ct_L.as<u32>(), n, ctx->ct_cptr.as<u64>()); CKL(); LAUNCHED(ctx);
+        if ((rc = exclusive_scan_inplace(ctx, ctx->ct_cptr.as<u64>(), n1))) return rc;
+        k_ct_layout<<<gn, 256, 0, st>>>(slot, col, f, base, n, ctx->ct_flag.as<u64>(), ctx->ct_cptr.as<u64>(), ctx->ct_start.as<u32>(), ctx->ct_pos.as<u32>(),
+            ctx->ct_next.as<uint8_t>(), rd, ctx->ct_read.as<int64_t>(), ctx->ct_rev.as<uint8_t>(), ctx->ct_beg.as<u32>(), ctx->ct_end.as<u32>(), ctx->ct_boff.as<u64>());
+        CKL(); LAUNCHED(ctx);
+        if ((rc = exclusive_scan_inplace(ctx, ctx->ct_boff.as<u64>(), n1))) return rc;
+        const u32 gc = (u32)std::min<u64>(gn, (u64)grid_for(ctx, 4));
+        k_og_count<<<gc, 256, 0, st>>>(ctx->ct_branch.as<uint8_t>(), n, d_cnt); CKL(); LAUNCHED(ctx);
+        k_og_count<<<gc, 256, 0, st>>>(ctx->ct_cyc.as<uint8_t>(), n, d_cnt + 1); CKL(); LAUNCHED(ctx);
+    }
+    // totals: contigs, reads in contigs, bases (the scans end at n: entries past the last contig / read are zero)
+    u64 h[5] = {0, 0, 0, 0, 0};
+    if (n) CK(cudaMemcpyAsync(&h[0], ctx->ct_flag.as<u64>() + n, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&h[1], ctx->ct_cptr.as<u64>() + n, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&h[2], ctx->ct_boff.as<u64>() + n, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&h[3], d_cnt, 16, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    elba_fe_contig_info_t I; std::memset(&I, 0, sizeof I);
+    I.ncontigs = h[0]; I.contig_reads = h[1]; I.bases = h[2]; I.branches = h[3]; I.cycles = h[4];
+    int64_t first = 0, count = 0;
+    elba_fe_block_extent((int64_t)I.ncontigs, nranks, rank, &first, &count);
+    I.first = (u64)first; I.count = (u64)count;
+    // this rank's block: bases and bytes per contig, byte offsets, then the packed sequences
+    const u64 c1 = I.count + 1;
+    CK(ctx->ct_blen.ensure(8 * c1)); CK(ctx->ct_bbyte.ensure(8 * c1));
+    k_ct_block<<<nblk(c1, 256), 256, 0, st>>>(ctx->ct_cptr.as<u64>(), ctx->ct_boff.as<u64>(), I.first, I.count, ctx->ct_blen.as<u64>(), ctx->ct_bbyte.as<u64>()); CKL(); LAUNCHED(ctx);
+    if ((rc = exclusive_scan_inplace(ctx, ctx->ct_bbyte.as<u64>(), c1))) return rc;
+    u64 b[3] = {0, 0, 0};
+    CK(cudaMemcpyAsync(&b[0], ctx->ct_bbyte.as<u64>() + I.count, 8, cudaMemcpyDeviceToHost, st));
+    u64 cp[2] = {0, 0};
+    CK(cudaMemcpyAsync(&cp[0], ctx->ct_cptr.as<u64>() + I.first, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&cp[1], ctx->ct_cptr.as<u64>() + I.first + I.count, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    CK(cudaMemcpyAsync(&b[1], ctx->ct_boff.as<u64>() + cp[0], 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&b[2], ctx->ct_boff.as<u64>() + cp[1], 8, cudaMemcpyDeviceToHost, st));
+    CK(ctx->ct_packed.ensure(b[0] + 64));
+    if (b[0])
+    {
+        k_ct_pack<<<nblk(b[0], 256), 256, 0, st>>>(ctx->ct_bbyte.as<u64>(), I.count, I.first, ctx->ct_cptr.as<u64>(), ctx->ct_boff.as<u64>(), ctx->ct_read.as<int64_t>(),
+            ctx->ct_rev.as<uint8_t>(), ctx->ct_beg.as<u32>(), ctx->ct_end.as<u32>(), base, rd, ctx->ct_packed.as<uint8_t>()); CKL(); LAUNCHED(ctx);
+    }
+    CK(cudaEventRecord(ctx->ct_e1, st));
+    CK(cudaStreamSynchronize(st));
+    I.my_bytes = b[0]; I.my_bases = b[2] - b[1];
+    float ms = 0; if (cudaEventElapsedTime(&ms, ctx->ct_e0, ctx->ct_e1) == cudaSuccess) I.ms = ms;
+    ctx->ct_info = I; ctx->ct_done = true;
+    if (info) *info = I;
+    return 0;
+}
+
+int elba_fe_contigs(elba_fe_ctx *ctx, elba_fe_contig_info_t *info)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->og_done || !ctx->tr_done || !ctx->tr_resident)
+        return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_contigs: needs the string graph of elba_fe_reduce_overlap_graph of the current overlap graph");
+    if (ctx->read_gen != ctx->xd_read_gen || ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_contigs: the reads changed after elba_fe_align");
+    const u64 Nt = ctx->og_nreads, m = ctx->tr_out;
+    if (Nt >= 0xFFFFFFF0ull || m >= 0xFFFFFFF0ull) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs: too many reads or string-graph entries");
+    CK(cudaSetDevice(ctx->cfg.device));
+    ctx->ct_done = false;
+    { int rcw = wait_reads(ctx); if (rcw) return rcw; }
+    CtReads rd;
+    if (ctx->comm.nranks > 1) { rd.buf = ctx->xa_buf.as<uint8_t>(); rd.off = ctx->xa_off.as<u64>(); rd.len = ctx->xa_len.as<u32>(); }
+    else { rd.buf = ctx->packed.as<uint8_t>(); rd.off = ctx->off.as<u64>(); rd.len = ctx->len32.as<u32>(); }
+    return contigs_device(ctx, ctx->tr_orow.as<int64_t>(), ctx->tr_ocol.as<int64_t>(), ctx->tr_of.as<int32_t>(), m, (u32)Nt, ctx->og_base, rd,
+                          ctx->comm.rank, std::max(ctx->comm.nranks, 1), info);
+}
+
+int elba_fe_contigs_from_graph(elba_fe_ctx *ctx, const int64_t *row, const int64_t *col, const int32_t *fields, uint64_t nnz, elba_fe_contig_info_t *info)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (ctx->phase < 1) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_contigs_from_graph: no reads resident");
+    if (nnz >= 0xFFFFFFF0ull) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: too many entries");
+    if (nnz && (!row || !col || !fields)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: null triples");
+    const int64_t base = ctx->read_id_offset, n = (int64_t)ctx->n;
+    // validate, and sort row-major: key = local row << 32 | local column
+    std::vector<std::pair<u64, u64>> key(nnz);
+    for (u64 e = 0; e < nnz; ++e)
+    {
+        if (row[e] < base || row[e] >= base + n || col[e] < base || col[e] >= base + n)
+            return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: read id outside this context's reads");
+        if (row[e] == col[e]) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: diagonal entry");
+        if (fields[4 * e] < 0 || fields[4 * e] > 3) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: direction outside 0..3");
+        key[e] = { ((u64)(row[e] - base) << 32) | (u64)(col[e] - base), e };
+    }
+    std::sort(key.begin(), key.end());
+    for (u64 e = 0; e < nnz; ++e)
+    {
+        if (e && key[e].first == key[e - 1].first) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: repeated coordinate");
+        const u64 mirror = (key[e].first << 32) | (key[e].first >> 32);
+        if (!std::binary_search(key.begin(), key.end(), std::make_pair(mirror, (u64)0), [](const std::pair<u64, u64> &a, const std::pair<u64, u64> &b) { return a.first < b.first; }))
+            return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_contigs_from_graph: not symmetric");
+    }
+    std::vector<int64_t> r(nnz), c(nnz); std::vector<int32_t> f(4 * nnz);
+    for (u64 e = 0; e < nnz; ++e)
+    {
+        const u64 s = key[e].second;
+        r[e] = row[s]; c[e] = col[s]; for (int j = 0; j < 4; ++j) f[4 * e + j] = fields[4 * s + j];
+    }
+    CK(cudaSetDevice(ctx->cfg.device));
+    ctx->ct_done = false;
+    { int rcw = wait_reads(ctx); if (rcw) return rcw; }
+    cudaStream_t st = ctx->stream;
+    CK(ctx->ct_in_row.ensure(8 * nnz + 8)); CK(ctx->ct_in_col.ensure(8 * nnz + 8)); CK(ctx->ct_in_f.ensure(16 * nnz + 16));
+    if (nnz)
+    {
+        CK(cudaMemcpyAsync(ctx->ct_in_row.p, r.data(), 8 * nnz, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(ctx->ct_in_col.p, c.data(), 8 * nnz, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(ctx->ct_in_f.p, f.data(), 16 * nnz, cudaMemcpyHostToDevice, st));
+    }
+    CtReads rd; rd.buf = ctx->packed.as<uint8_t>(); rd.off = ctx->off.as<u64>(); rd.len = ctx->len32.as<u32>();
+    return contigs_device(ctx, ctx->ct_in_row.as<int64_t>(), ctx->ct_in_col.as<int64_t>(), ctx->ct_in_f.as<int32_t>(), nnz, ctx->n, base, rd, 0, 1, info);
+}
+
+int elba_fe_get_contig_layout(elba_fe_ctx *ctx, uint64_t *ptr, int64_t *read, uint8_t *reverse, uint32_t *beg, uint32_t *end)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->ct_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_get_contig_layout: call elba_fe_contigs first");
+    CK(cudaSetDevice(ctx->cfg.device));
+    const u64 C = ctx->ct_info.ncontigs, R = ctx->ct_info.contig_reads;
+    if (ptr && C) D2H(ptr, ctx->ct_cptr.p, 8 * (C + 1));
+    if (ptr && !C) ptr[0] = 0;
+    D2H(read, ctx->ct_read.p, 8 * R); D2H(reverse, ctx->ct_rev.p, R); D2H(beg, ctx->ct_beg.p, 4 * R); D2H(end, ctx->ct_end.p, 4 * R);
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int elba_fe_get_contigs(elba_fe_ctx *ctx, uint8_t *packed, uint64_t *byte_off, uint64_t *len)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->ct_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_get_contigs: call elba_fe_contigs first");
+    CK(cudaSetDevice(ctx->cfg.device));
+    const u64 K = ctx->ct_info.count;
+    D2H(packed, ctx->ct_packed.p, ctx->ct_info.my_bytes); D2H(byte_off, ctx->ct_bbyte.p, 8 * K); D2H(len, ctx->ct_blen.p, 8 * K);
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int elba_fe_device_contigs(elba_fe_ctx *ctx, const uint8_t **packed, const uint64_t **byte_off, const uint64_t **len)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->ct_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_device_contigs: call elba_fe_contigs first");
+    if (packed) *packed = ctx->ct_packed.as<uint8_t>();
+    if (byte_off) *byte_off = ctx->ct_bbyte.as<uint64_t>();
+    if (len) *len = ctx->ct_blen.as<uint64_t>();
     return 0;
 }
 

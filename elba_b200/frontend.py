@@ -55,6 +55,35 @@ class Timings(C.Structure):
         return {n: (int(getattr(self, n)) if n == "kernel_launches" else float(getattr(self, n))) for n, _ in self._fields_}
 
 
+class ContigInfo(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("ncontigs", "contig_reads", "bases", "branches", "cycles", "first", "count", "my_bases", "my_bytes")] + \
+               [("ms", C.c_float), ("reserved", C.c_float)]
+
+    def as_dict(self):
+        return {n: (float(getattr(self, n)) if n == "ms" else int(getattr(self, n))) for n, _ in self._fields_ if n != "reserved"}
+
+
+@dataclass
+class Contigs:
+    """What elba_fe_contigs leaves: the whole job's layout (contig c = entries ptr[c] .. ptr[c + 1] of read, reverse, beg, end) and
+    this rank's block of contigs [info["first"], + info["count"]) as packed sequences."""
+    info: dict
+    ptr: np.ndarray
+    read: np.ndarray
+    reverse: np.ndarray
+    beg: np.ndarray
+    end: np.ndarray
+    seqs: DnaBuffer
+
+
+def write_contigs_fa(path: str, seqs: DnaBuffer, first: int = 0, mode: str = "w"):
+    """Write contigs as FASTA (`.contigs.fa`): one record `>contig_<id>` per contig, the sequence on one line; ids count from
+    `first` (a rank's block appends with mode "a" and its own first id)."""
+    with open(path, mode) as fa:
+        for i in range(seqs.size()):
+            fa.write(f">contig_{first + i}\n{seqs.read_ascii(i)}\n")
+
+
 # every symbol include/elba_fe.h declares (tests check the library exports all of them)
 ABI_SYMBOLS = (
     "elba_fe_default_config", "elba_fe_create", "elba_fe_destroy", "elba_fe_last_error", "elba_fe_version", "elba_fe_set_stream",
@@ -67,6 +96,7 @@ ABI_SYMBOLS = (
     "elba_fe_transitive_reduction", "elba_fe_get_string_graph",
     "elba_fe_overlap_graph", "elba_fe_get_overlap_graph", "elba_fe_reduce_overlap_graph",
     "elba_fe_ingest_fasta", "elba_fe_reads_size", "elba_fe_get_reads", "elba_fe_B_dcsc", "elba_fe_get_B_dcsc", "elba_fe_device_B_dcsc",
+    "elba_fe_contigs", "elba_fe_contigs_from_graph", "elba_fe_get_contig_layout", "elba_fe_get_contigs", "elba_fe_device_contigs",
 )
 
 _lib = None
@@ -329,6 +359,33 @@ class Context:
         osrc, otr = np.zeros(m, np.uint64), np.zeros(m, np.uint8)
         self._ck(self.L.elba_fe_get_string_graph(self.h, _p(orow), _p(ocol), _p(of), _p(osrc), _p(otr)))
         return orow, ocol, of, osrc, otr
+
+    def _contigs_result(self, info: ContigInfo) -> Contigs:
+        d = info.as_dict()
+        nc, nr, k = d["ncontigs"], d["contig_reads"], d["count"]
+        ptr, read, rev = np.zeros(nc + 1, np.uint64), np.zeros(nr, np.int64), np.zeros(nr, np.uint8)
+        beg, end = np.zeros(nr, np.uint32), np.zeros(nr, np.uint32)
+        self._ck(self.L.elba_fe_get_contig_layout(self.h, _p(ptr), _p(read), _p(rev), _p(beg), _p(end)))
+        packed, off, lens = np.zeros(d["my_bytes"], np.uint8), np.zeros(k, np.uint64), np.zeros(k, np.uint64)
+        self._ck(self.L.elba_fe_get_contigs(self.h, _p(packed), _p(off), _p(lens)))
+        return Contigs(d, ptr, read, rev, beg, end, DnaBuffer(packed, off, lens))
+
+    def contigs(self) -> Contigs:
+        """Contigs from the string graph string_graph() left on the device (elba_fe_contigs; the rule is in include/elba_fe.h):
+        the whole job's layout and this rank's block of sequences."""
+        info = ContigInfo()
+        self._ck(self.L.elba_fe_contigs(self.h, C.byref(info)))
+        return self._contigs_result(info)
+
+    def contigs_from_graph(self, rows, cols, fields) -> Contigs:
+        """The same from a string graph given on the host (elba_fe_contigs_from_graph) over this context's own reads:
+        (rows, cols, fields[nnz, 4] = direction, directionT, suffix, suffixT) with global read ids."""
+        rows, cols = np.ascontiguousarray(rows, np.int64), np.ascontiguousarray(cols, np.int64)
+        fields = np.ascontiguousarray(fields, np.int32).reshape(-1, 4)
+        info = ContigInfo()
+        self._ck(self.L.elba_fe_contigs_from_graph(self.h, _p(rows) if len(rows) else None, _p(cols) if len(rows) else None,
+                                                   _p(fields) if len(rows) else None, C.c_uint64(len(rows)), C.byref(info)))
+        return self._contigs_result(info)
 
     def hll(self):
         regs, est = np.zeros(4096, np.uint8), C.c_double()

@@ -252,6 +252,40 @@ int elba_fe_get_overlap_graph(elba_fe_ctx *ctx, int64_t *row, int64_t *col, int3
                               int32_t *src_rank, uint64_t *src_pair);
 int elba_fe_reduce_overlap_graph(elba_fe_ctx *ctx, int32_t fuzz, uint64_t *nnz_out);
 
+/* ---- contigs from the string graph (the stage GenerateContigs runs in the reference, src/main.cpp:320) -------------------
+ * The rule (DESIGN.md §3d; restated in tests/contig_inputs.py; parity with the reference's own contig output is UNPINNED):
+ * entry e = (i, j) of S has t(e) = (dir >> 1) & 1, the end of read i it leaves from (0 = 3' end, 1 = 5' start), and suffix =
+ * the bases j adds beyond i.  A read is a branch if its row of S has more than two entries, or two with the same t.  The
+ * chain graph G = the entries of S between two reads that are not branches (and whose mirror is in S); every component of G
+ * with two or more reads is a path or a cycle and gives one contig.  A path starts at the smaller of its two end reads; a cycle
+ * at its smallest read s, first towards the smaller of s's two neighbours (the edge to the other one is cut; counted in
+ * cycles).  On the walk v0 .. vm, v_k (k < m) is forward iff t(v_k -> v_k+1) == 0 and vm iff t(vm -> vm-1) == 1; v0 adds
+ * [0, len), v_k (k >= 1) with s = clamp(suffix(v_k-1 -> v_k), 0, len) adds [len - s, len) forward or [0, s) reverse-complemented.
+ * Contigs are numbered in ascending order of their start read's global id, whatever the number of GPUs.
+ * contigs: from the S that elba_fe_reduce_overlap_graph left on the device for the current R, and the reads elba_fe_align saw
+ *   (ELBA_FE_ERR_STATE otherwise: a host-route elba_fe_transitive_reduction, reads replaced after align).  No collective:
+ *   every rank builds the whole layout and the sequences of its block of contigs, elba_fe_block_extent(ncontigs, nranks, rank).
+ * contigs_from_graph: S from the host in the layout of elba_fe_get_string_graph over this context's own reads (global ids in
+ *   [read_id_offset, read_id_offset + nreads)); checked on the host: ids, dir in 0..3, no diagonal, distinct coordinates,
+ *   symmetric coordinates (ELBA_FE_ERR_INVALID otherwise).  No collective; builds every contig.
+ * get_contig_layout: the whole job: ptr[ncontigs + 1] into the contig_reads arrays read (global id), reverse (1 = reverse
+ *   complemented), beg / end (the segment [beg, end) of the read, before reverse complementing); any pointer may be NULL.
+ * get_contigs / device_contigs: this rank's block as a DnaBuffer: 2-bit packed, every contig byte-aligned at byte_off[count],
+ *   len[count] bases (u64 both: the device arrays can go straight into elba_fe_set_reads_device of another context).
+ * Calls that discard R or replace S or the reads discard the contigs: the getters are ELBA_FE_ERR_STATE until the next call. */
+typedef struct {
+    uint64_t ncontigs, contig_reads, bases;    /* whole job */
+    uint64_t branches, cycles;
+    uint64_t first, count, my_bases, my_bytes; /* this rank's block of contigs */
+    float ms; float reserved;                  /* device time of the call */
+} elba_fe_contig_info_t;
+int elba_fe_contigs(elba_fe_ctx *ctx, elba_fe_contig_info_t *info);
+int elba_fe_contigs_from_graph(elba_fe_ctx *ctx, const int64_t *row, const int64_t *col, const int32_t *fields /* nnz x 4 */, uint64_t nnz,
+                               elba_fe_contig_info_t *info);
+int elba_fe_get_contig_layout(elba_fe_ctx *ctx, uint64_t *ptr /* ncontigs + 1 */, int64_t *read, uint8_t *reverse, uint32_t *beg, uint32_t *end);
+int elba_fe_get_contigs(elba_fe_ctx *ctx, uint8_t *packed, uint64_t *byte_off, uint64_t *len);
+int elba_fe_device_contigs(elba_fe_ctx *ctx, const uint8_t **packed, const uint64_t **byte_off, const uint64_t **len);
+
 /* ---- the reference's sizing sketches, bit-exact (not needed for the result when lower >= 2) ----------- */
 /* HyperLogLog over the canonical k-mers of the uploaded reads exactly as KmerEstimateHandler drives it
  * (include/KmerOps.hpp:58-69, src/HyperLogLog.cpp:40-76): registers[4096] and estimate(). */
