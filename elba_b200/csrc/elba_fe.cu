@@ -16,6 +16,7 @@
 #include "transitive.cuh"
 #include "overlap_graph.cuh"
 #include "contigs.cuh"
+#include "paf.cuh"
 #include "comm.cuh"
 #include <cub/cub.cuh>
 #include <string>
@@ -121,6 +122,10 @@ struct elba_fe_ctx
     DevBuf ct_in_row, ct_in_col, ct_in_f, ct_ptr, ct_branch, ct_slot, ct_succ[2], ct_dist[2], ct_mn[2], ct_cyc, ct_flag, ct_start, ct_pos, ct_next, ct_L,
            ct_cptr, ct_read, ct_rev, ct_beg, ct_end, ct_boff, ct_blen, ct_bbyte, ct_packed;
     elba_fe_contig_info_t ct_info; bool ct_done = false; cudaEvent_t ct_e0 = nullptr, ct_e1 = nullptr;
+    // elba_fe_paf: read names of the job (char arena + offsets), line lengths / offsets, string-graph lines, the text of this rank
+    DevBuf pf_names, pf_noff, pf_len, pf_flag, pf_q, pf_t, pf_dir, pf_v, pf_text;
+    u64 pf_nnames = 0; bool pf_has_names = false;
+    elba_fe_paf_info_t pf_info; bool pf_done = false; cudaEvent_t pf_e0 = nullptr, pf_e1 = nullptr;
     DevBuf fa_raw, fa_rec, fa_items;                       // elba_fe_ingest_fasta: the raw FASTA chunk, its .fai records, first work item of every read
     DevBuf dc_key, dc_key2, dc_val, dc_val2, dc_head, dc_jc, dc_cp, dc_ir, dc_num, dc_seeds; u64 dc_nzc = 0; bool dc_built = false;      // B by column (DCSC)
     // multi-GPU
@@ -315,6 +320,7 @@ int elba_fe_create(const elba_fe_config *cfg, elba_fe_ctx **out)
     cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming); cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming);
     cudaEventCreate(&ctx->ev_x0); cudaEventCreate(&ctx->ev_x1); cudaEventCreate(&ctx->xd_e0); cudaEventCreate(&ctx->xd_e1);
     cudaEventCreate(&ctx->og_e0); cudaEventCreate(&ctx->og_e1); cudaEventCreate(&ctx->ct_e0); cudaEventCreate(&ctx->ct_e1);
+    cudaEventCreate(&ctx->pf_e0); cudaEventCreate(&ctx->pf_e1);
     if (ctx->tmp64.ensure(8192) != cudaSuccess || ctx->ctr.ensure(128) != cudaSuccess) { elba_fe_destroy(ctx); return fail(nullptr, ELBA_FE_ERR_OOM, "cudaMalloc failed"); }
     if (const char *e = getenv("ELBA_FE_TRACE")) ctx->trace = atoi(e) != 0;
     if (const char *e = getenv("ELBA_FE_SCRATCH_MB")) { long v = atol(e); if (v >= 8 && v <= 65536) ctx->scratch_mb = (u64)v; }
@@ -348,7 +354,8 @@ int elba_fe_destroy(elba_fe_ctx *ctx)
         &ctx->xa_buf, &ctx->xa_off, &ctx->xa_len,
         &ctx->ct_in_row, &ctx->ct_in_col, &ctx->ct_in_f, &ctx->ct_ptr, &ctx->ct_branch, &ctx->ct_slot, &ctx->ct_succ[0], &ctx->ct_succ[1], &ctx->ct_dist[0], &ctx->ct_dist[1],
         &ctx->ct_mn[0], &ctx->ct_mn[1], &ctx->ct_cyc, &ctx->ct_flag, &ctx->ct_start, &ctx->ct_pos, &ctx->ct_next, &ctx->ct_L, &ctx->ct_cptr, &ctx->ct_read, &ctx->ct_rev,
-        &ctx->ct_beg, &ctx->ct_end, &ctx->ct_boff, &ctx->ct_blen, &ctx->ct_bbyte, &ctx->ct_packed, &ctx->fa_raw, &ctx->fa_rec, &ctx->fa_items, &ctx->dc_key, &ctx->dc_key2, &ctx->dc_val, &ctx->dc_val2, &ctx->dc_head, &ctx->dc_jc, &ctx->dc_cp, &ctx->dc_ir, &ctx->dc_num, &ctx->dc_seeds,
+        &ctx->ct_beg, &ctx->ct_end, &ctx->ct_boff, &ctx->ct_blen, &ctx->ct_bbyte, &ctx->ct_packed,
+        &ctx->pf_names, &ctx->pf_noff, &ctx->pf_len, &ctx->pf_flag, &ctx->pf_q, &ctx->pf_t, &ctx->pf_dir, &ctx->pf_v, &ctx->pf_text, &ctx->fa_raw, &ctx->fa_rec, &ctx->fa_items, &ctx->dc_key, &ctx->dc_key2, &ctx->dc_val, &ctx->dc_val2, &ctx->dc_head, &ctx->dc_jc, &ctx->dc_cp, &ctx->dc_ir, &ctx->dc_num, &ctx->dc_seeds,
         &ctx->plan, &ctx->bfill, &ctx->ovf, &ctx->scratch[0], &ctx->scratch[1], &ctx->skm_slab, &ctx->skm_fill, &ctx->skm_ovf, &ctx->seeds, &ctx->perm, &ctx->rel_idx, &ctx->rel_idx_s,
         &ctx->recvbuf, &ctx->recvcnt, &ctx->tmp64, &ctx->rel_all_key, &ctx->rel_all_cnt, &ctx->g_key, &ctx->g_pos, &ctx->pack_key, &ctx->l_rowptr, &ctx->l_col,
         &ctx->r_key, &ctx->r_key2, &ctx->r_pos, &ctx->r_colptr, &ctx->r_row, &ctx->r_ptr };
@@ -371,6 +378,8 @@ int elba_fe_destroy(elba_fe_ctx *ctx)
     if (ctx->og_e1) cudaEventDestroy(ctx->og_e1);
     if (ctx->ct_e0) cudaEventDestroy(ctx->ct_e0);
     if (ctx->ct_e1) cudaEventDestroy(ctx->ct_e1);
+    if (ctx->pf_e0) cudaEventDestroy(ctx->pf_e0);
+    if (ctx->pf_e1) cudaEventDestroy(ctx->pf_e1);
     delete ctx;
     return 0;
 }
@@ -401,7 +410,7 @@ static int stage_reads(elba_fe_ctx *ctx, const uint8_t *packed, uint64_t packed_
     if (nreads && (!byte_off || !len)) return fail(ctx, ELBA_FE_ERR_INVALID, "null read tables");
     if (packed_bytes && !packed) return fail(ctx, ELBA_FE_ERR_INVALID, "null arena");
     CK(cudaSetDevice(ctx->cfg.device));
-    ctx->phase = 0; ++ctx->read_gen; ctx->ct_done = false;
+    ctx->phase = 0; ++ctx->read_gen; ctx->ct_done = ctx->pf_done = false;
     ctx->n = (u32)nreads; ctx->packed_bytes = packed_bytes; ctx->read_id_offset = read_id_offset;
     cudaStream_t st = ctx->stream;
     CK(cudaEventRecord(ctx->ev[0], st));
@@ -503,7 +512,7 @@ int elba_fe_ingest_fasta(elba_fe_ctx *ctx, const char *chunk, uint64_t chunk_byt
         head += nb; nitems += (nb + FI_ITEM_BYTES - 1) / FI_ITEM_BYTES;
     }
     off[nreads] = head; items[nreads] = nitems;
-    ctx->phase = 0; ++ctx->read_gen; ctx->ct_done = false;
+    ctx->phase = 0; ++ctx->read_gen; ctx->ct_done = ctx->pf_done = false;
     ctx->n = (u32)nreads; ctx->packed_bytes = head; ctx->read_id_offset = read_id_offset; ctx->up_n = 0;
     cudaStream_t st = ctx->stream;
     CK(cudaEventRecord(ctx->ev[0], st));
@@ -987,7 +996,7 @@ int elba_fe_count(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 1) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_count: no reads uploaded");
-    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = ctx->pf_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     const int k = ctx->cfg.k, stride = ctx->cfg.stride; const u32 lower = ctx->cfg.lower, upper = ctx->cfg.upper;
     cudaStream_t st = ctx->stream;
@@ -1458,7 +1467,7 @@ int elba_fe_build_A(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 2) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_build_A: call elba_fe_count first");
-    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = ctx->pf_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     ReadsView rv = view(ctx);
@@ -1647,7 +1656,7 @@ int elba_fe_spgemm(elba_fe_ctx *ctx)
 {
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 3) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_spgemm: call elba_fe_build_A first");
-    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = ctx->pf_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     const u32 N = ctx->op.l_rows; const u64 nnzA = ctx->op.l_nnz;       // rows of this GPU's block of B
@@ -2098,7 +2107,7 @@ int elba_fe_align(elba_fe_ctx *ctx, int mat, int mis, int gap, int dropoff, uint
     if (!ctx) return ELBA_FE_ERR_INVALID;
     if (ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_align: call elba_fe_spgemm first");
     if (mat <= 0 || mis > 0 || gap >= 0 || dropoff < 0) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_align: need mat > 0, mis <= 0, gap < 0, dropoff >= 0");
-    ctx->og_aligned = ctx->og_done = ctx->ct_done = false;
+    ctx->og_aligned = ctx->og_done = ctx->ct_done = ctx->pf_done = false;
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
     const u64 nnz = ctx->sz.nnzB; const u32 N = ctx->b_rows;
@@ -2275,7 +2284,7 @@ int elba_fe_transitive_reduction(elba_fe_ctx *ctx, const int64_t *row, const int
     }
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
-    ctx->tr_done = ctx->tr_resident = ctx->ct_done = false; ctx->tr_out = 0;
+    ctx->tr_done = ctx->tr_resident = ctx->ct_done = ctx->pf_done = false; ctx->tr_out = 0;
     CK(cudaEventRecord(ctx->ev[0], st));
     if (nnz)
     {
@@ -2294,7 +2303,7 @@ int elba_fe_overlap_graph(elba_fe_ctx *ctx, uint64_t *nnz, uint64_t *ncontained)
     if (!ctx->og_aligned || !ctx->xd_done || ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_overlap_graph: call elba_fe_align first");
     CK(cudaSetDevice(ctx->cfg.device));
     cudaStream_t st = ctx->stream;
-    ctx->og_done = ctx->tr_resident = ctx->ct_done = false;
+    ctx->og_done = ctx->tr_resident = ctx->ct_done = ctx->pf_done = false;
     const int W = ctx->comm.nranks;
     const u64 np = ctx->xd_pairs, Nt = W > 1 ? ctx->N_total : (u64)ctx->n;
     // job-relative id of this block's first row / column read (one GPU: 0)
@@ -2382,7 +2391,7 @@ int elba_fe_reduce_overlap_graph(elba_fe_ctx *ctx, int32_t fuzz, uint64_t *nnz_o
     if (Nt >= 0xFFFFFFF0ull) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_reduce_overlap_graph: too many reads");
     if (nnz >= (1ull << 31)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_reduce_overlap_graph: more than 2^31 overlaps");
     CK(cudaSetDevice(ctx->cfg.device));
-    ctx->tr_done = ctx->ct_done = false; ctx->tr_out = 0;
+    ctx->tr_done = ctx->ct_done = ctx->pf_done = false; ctx->tr_out = 0;
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
     const int rc = tr_reduce_device(ctx, ctx->og_row.as<int64_t>(), ctx->og_col.as<int64_t>(), ctx->og_f.as<int32_t>(), nnz, (u32)Nt, fuzz, ctx->og_base, nnz_out);
     if (rc == 0) ctx->tr_resident = true;
@@ -2589,6 +2598,150 @@ int elba_fe_device_contigs(elba_fe_ctx *ctx, const uint8_t **packed, const uint6
     if (packed) *packed = ctx->ct_packed.as<uint8_t>();
     if (byte_off) *byte_off = ctx->ct_bbyte.as<uint64_t>();
     if (len) *len = ctx->ct_blen.as<uint64_t>();
+    return 0;
+}
+
+// ---- PAF text of the overlap graph and of the string graph (paf.cuh): the files src/main.cpp:303,317 write -----------------
+int elba_fe_set_read_names(elba_fe_ctx *ctx, const char *names, const uint64_t *name_off, uint64_t nreads)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (nreads && (!names || !name_off)) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_set_read_names: null names");
+    if (nreads >= 0xFFFFFFF0ull) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_set_read_names: too many reads");
+    for (u64 r = 0; r < nreads; ++r)
+        if (name_off[r + 1] <= name_off[r]) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_set_read_names: empty name (offsets must increase)");
+    const u64 b0 = nreads ? name_off[0] : 0, nb = nreads ? name_off[nreads] - b0 : 0;
+    for (u64 b = 0; b < nb; ++b)
+        if ((unsigned char)names[b0 + b] <= 0x20) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_set_read_names: a name holds a byte <= 0x20 (blank or control)");
+    CK(cudaSetDevice(ctx->cfg.device));
+    ctx->pf_done = ctx->pf_has_names = false; ctx->pf_nnames = 0;
+    if (!nreads) return 0;
+    std::vector<u64> off(nreads + 1);
+    for (u64 r = 0; r <= nreads; ++r) off[r] = name_off[r] - b0;
+    CK(ctx->pf_names.ensure(nb + 16)); CK(ctx->pf_noff.ensure(8 * (nreads + 1)));
+    CK(cudaMemcpyAsync(ctx->pf_names.p, names + b0, nb, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->pf_noff.p, off.data(), 8 * (nreads + 1), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->pf_has_names = true; ctx->pf_nnames = nreads;
+    return 0;
+}
+
+// the n lines of s: lengths and offsets, then the text of lines [first, first + count) into pf_text.
+// h = {offset of line first, bytes of lines [first, first + count), bytes of all n lines}
+static int paf_text(elba_fe_ctx *ctx, const PafSrc &s, u64 n, u64 first, u64 count, u64 h[3])
+{
+    cudaStream_t st = ctx->stream;
+    int rc;
+    CK(ctx->pf_len.ensure(8 * (n + 1)));
+    u64 *off = ctx->pf_len.as<u64>();
+    k_paf_len<<<nblk(n + 1, 256), 256, 0, st>>>(s, n, off); CKL(); LAUNCHED(ctx);
+    if ((rc = exclusive_scan_inplace(ctx, off, n + 1))) return rc;
+    u64 b[3] = {0, 0, 0};
+    CK(cudaMemcpyAsync(&b[0], off + first, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&b[1], off + first + count, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(&b[2], off + n, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    h[0] = b[0]; h[1] = b[1] - b[0]; h[2] = b[2];
+    CK(ctx->pf_text.ensure(h[1] + 16));
+    if (count) { k_paf_write<<<nblk(count, PAF_THREADS), PAF_THREADS, 0, st>>>(s, off, first, count, ctx->pf_text.as<char>()); CKL(); LAUNCHED(ctx); }
+    return 0;
+}
+
+int elba_fe_paf(elba_fe_ctx *ctx, int which, elba_fe_paf_info_t *info)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (which != ELBA_FE_PAF_OVERLAP && which != ELBA_FE_PAF_STRING) return fail(ctx, ELBA_FE_ERR_INVALID, "elba_fe_paf: which must be ELBA_FE_PAF_OVERLAP or ELBA_FE_PAF_STRING");
+    if (!ctx->og_aligned || !ctx->xd_done || ctx->phase < 4) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_paf: call elba_fe_align first");
+    if (which == ELBA_FE_PAF_STRING)
+    {
+        if (!ctx->og_done || !ctx->tr_done || !ctx->tr_resident)
+            return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_paf: needs the string graph of elba_fe_reduce_overlap_graph of the current overlap graph");
+        if (ctx->read_gen != ctx->xd_read_gen) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_paf: the reads changed after elba_fe_align");
+    }
+    const int W = std::max(ctx->comm.nranks, 1), me = ctx->comm.rank;
+    const u64 Nt = W > 1 ? ctx->N_total : (u64)ctx->n;
+    if (ctx->pf_has_names && ctx->pf_nnames != Nt) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_paf: the read names are not those of the job's reads (count differs)");
+    CK(cudaSetDevice(ctx->cfg.device));
+    ctx->pf_done = false;
+    { int rcw = wait_reads(ctx); if (rcw) return rcw; }
+    cudaStream_t st = ctx->stream;
+    int rc;
+    CK(cudaEventRecord(ctx->pf_e0, st));
+    PafSrc s;
+    s.len = W > 1 ? ctx->xa_len.as<u32>() : ctx->len32.as<u32>();
+    s.names = ctx->pf_has_names ? ctx->pf_names.as<char>() : nullptr; s.name_off = ctx->pf_noff.as<u64>(); s.id_base = ctx->read_base0;
+    elba_fe_paf_info_t I; std::memset(&I, 0, sizeof I);
+    u64 h[3];
+    if (which == ELBA_FE_PAF_OVERLAP)
+    {
+        // this rank's alignments, in the order of elba_fe_get_alignments; the ranks' parts follow in rank order
+        const u64 np = ctx->xd_pairs;
+        s.q = ctx->xd_prow.as<u32>(); s.t = ctx->xd_pcol.as<u32>();
+        s.qbase = (u32)(ctx->op.row0 - ctx->read_base0); s.tbase = (u32)(ctx->op.col0 - ctx->read_base0);
+        s.v = ctx->xd_out.as<int32_t>(); s.vstride = PAF_XD_FIELDS; s.dir = ctx->xd_out.as<int32_t>() + OG_DIR; s.dstride = PAF_XD_FIELDS;
+        if ((rc = paf_text(ctx, s, np, 0, np, h))) return rc;
+        I.lines = np; I.bytes = h[1];
+        std::vector<u64> bytes, lines;
+        if ((rc = allgather_u64(ctx, I.bytes, bytes))) return rc;
+        if ((rc = allgather_u64(ctx, I.lines, lines))) return rc;
+        for (int r = 0; r < W; ++r)
+        {
+            if (r < me) I.offset += bytes[r];
+            I.total_bytes += bytes[r]; I.total_lines += lines[r];
+        }
+    }
+    else
+    {
+        // lines = the entries of S with transposed == 0, in S's order; the printed fields come from the source alignment, which
+        // one rank holds: every rank fills those of its own, the others are zero, and one sum all-reduce completes them
+        const u64 m = ctx->tr_out;
+        CK(ctx->pf_flag.ensure(8 * (m + 1)));
+        k_paf_flags<<<nblk(m + 1, 256), 256, 0, st>>>(ctx->tr_otr.as<uint8_t>(), m, ctx->pf_flag.as<u64>()); CKL(); LAUNCHED(ctx);
+        if ((rc = exclusive_scan_inplace(ctx, ctx->pf_flag.as<u64>(), m + 1))) return rc;
+        u64 L = 0;
+        CK(cudaMemcpyAsync(&L, ctx->pf_flag.as<u64>() + m, 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        const u64 L1 = std::max<u64>(L, 1);
+        CK(ctx->pf_q.ensure(4 * L1)); CK(ctx->pf_t.ensure(4 * L1)); CK(ctx->pf_dir.ensure(4 * L1)); CK(ctx->pf_v.ensure(24 * L1));
+        u64 r_lo = 0;
+        for (int r = 0; r < me; ++r) r_lo += ctx->og_counts[r];
+        const u64 r_hi = r_lo + ctx->og_counts[me];
+        if (m)
+        {
+            k_paf_string_lines<<<nblk(m, 256), 256, 0, st>>>(ctx->tr_otr.as<uint8_t>(), ctx->pf_flag.as<u64>(), m, ctx->tr_orow.as<int64_t>(), ctx->tr_ocol.as<int64_t>(),
+                ctx->tr_of.as<int32_t>(), ctx->tr_osrc.as<u64>(), ctx->og_base, ctx->og_src.as<u64>(), r_lo, r_hi, ctx->xd_out.as<int32_t>(),
+                ctx->pf_q.as<u32>(), ctx->pf_t.as<u32>(), ctx->pf_dir.as<int32_t>(), ctx->pf_v.as<int32_t>()); CKL(); LAUNCHED(ctx);
+        }
+        if (W > 1 && L) NC(ctx->comm.api->AllReduce(ctx->pf_v.p, ctx->pf_v.p, (size_t)(6 * L), ncclInt32, ncclSum, ctx->comm.comm, st));
+        s.q = ctx->pf_q.as<u32>(); s.t = ctx->pf_t.as<u32>(); s.qbase = s.tbase = 0;
+        s.v = ctx->pf_v.as<int32_t>(); s.vstride = 6; s.dir = ctx->pf_dir.as<int32_t>(); s.dstride = 1;
+        int64_t first = 0, count = 0;
+        elba_fe_block_extent((int64_t)L, W, me, &first, &count);
+        if ((rc = paf_text(ctx, s, L, (u64)first, (u64)count, h))) return rc;
+        I.lines = (u64)count; I.bytes = h[1]; I.offset = h[0]; I.total_lines = L; I.total_bytes = h[2];
+    }
+    CK(cudaEventRecord(ctx->pf_e1, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0; if (cudaEventElapsedTime(&ms, ctx->pf_e0, ctx->pf_e1) == cudaSuccess) I.ms = ms;
+    ctx->pf_info = I; ctx->pf_done = true;
+    if (info) *info = I;
+    return 0;
+}
+
+int elba_fe_get_paf(elba_fe_ctx *ctx, char *text)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->pf_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_get_paf: call elba_fe_paf first");
+    CK(cudaSetDevice(ctx->cfg.device));
+    D2H(text, ctx->pf_text.p, ctx->pf_info.bytes);
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int elba_fe_device_paf(elba_fe_ctx *ctx, const char **text)
+{
+    if (!ctx) return ELBA_FE_ERR_INVALID;
+    if (!ctx->pf_done) return fail(ctx, ELBA_FE_ERR_STATE, "elba_fe_device_paf: call elba_fe_paf first");
+    if (text) *text = ctx->pf_text.as<char>();
     return 0;
 }
 

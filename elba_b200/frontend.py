@@ -84,6 +84,72 @@ def write_contigs_fa(path: str, seqs: DnaBuffer, first: int = 0, mode: str = "w"
             fa.write(f">contig_{first + i}\n{seqs.read_ascii(i)}\n")
 
 
+def write_at(path: str, data: bytes, offset: int, total: int, dist=None):
+    """One file written by every rank at once: rank 0 creates it and sets its size to `total` bytes, then (after a barrier) every
+    rank writes its `data` at `offset` with os.pwrite; returns when every rank's part is in.  `dist`: an initialised
+    torch.distributed, or None for one process."""
+    rank = dist.get_rank() if dist is not None else 0
+    if rank == 0:
+        fd = os.open(path, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o644)
+        os.ftruncate(fd, total)
+        os.close(fd)
+    if dist is not None:
+        dist.barrier()
+    fd = os.open(path, os.O_WRONLY)
+    try:
+        view, pos = memoryview(data), 0
+        while pos < len(view):
+            pos += os.pwrite(fd, view[pos:], offset + pos)
+    finally:
+        os.close(fd)
+    if dist is not None:
+        dist.barrier()
+
+
+def write_contigs_fa_parallel(path: str, seqs: DnaBuffer, first: int = 0, dist=None):
+    """The `.contigs.fa` of write_contigs_fa(path, all contigs) written by every rank at once: each rank's block of contigs
+    (ids from `first`) goes to its byte offset, found by all-gathering the ranks' byte counts over `dist` (torch.distributed)."""
+    data = "".join(f">contig_{first + i}\n{seqs.read_ascii(i)}\n" for i in range(seqs.size())).encode()
+    sizes = [len(data)]
+    if dist is not None:
+        sizes = [None] * dist.get_world_size()
+        dist.all_gather_object(sizes, len(data))
+    rank = dist.get_rank() if dist is not None else 0
+    write_at(path, data, sum(sizes[:rank]), sum(sizes), dist)
+
+
+PAF_OVERLAP, PAF_STRING = 0, 1
+
+
+class PafInfo(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in ("lines", "bytes", "offset", "total_lines", "total_bytes")] + [("ms", C.c_float), ("reserved", C.c_float)]
+
+    def as_dict(self):
+        return {n: (float(getattr(self, n)) if n == "ms" else int(getattr(self, n))) for n, _ in self._fields_ if n != "reserved"}
+
+
+def check_read_names(names):
+    """The names as bytes, checked as elba_fe_set_read_names checks them: every name non-empty, no byte <= 0x20 (PAF columns are
+    tab-separated and a FASTA name ends at the first blank).  Raises ValueError."""
+    out = []
+    for i, n in enumerate(names):
+        b = n.encode() if isinstance(n, str) else bytes(n)
+        if not b:
+            raise ValueError(f"read name {i} is empty")
+        if min(b) <= 0x20:
+            raise ValueError(f"read name {i} ({b[:40]!r}) holds a blank or control byte")
+        out.append(b)
+    return out
+
+
+def write_paf(path: str, ctx: "Context", which: int, dist=None) -> dict:
+    """`<prefix>.overlap.paf` (which = PAF_OVERLAP) or `.string.paf` (PAF_STRING) formatted on the device (Context.paf) and
+    written by every rank at its offset into one file; collective on several GPUs.  Returns the info dict."""
+    text, info = ctx.paf(which)
+    write_at(path, text, info["offset"], info["total_bytes"], dist)
+    return info
+
+
 # every symbol include/elba_fe.h declares (tests check the library exports all of them)
 ABI_SYMBOLS = (
     "elba_fe_default_config", "elba_fe_create", "elba_fe_destroy", "elba_fe_last_error", "elba_fe_version", "elba_fe_set_stream",
@@ -97,6 +163,7 @@ ABI_SYMBOLS = (
     "elba_fe_overlap_graph", "elba_fe_get_overlap_graph", "elba_fe_reduce_overlap_graph",
     "elba_fe_ingest_fasta", "elba_fe_reads_size", "elba_fe_get_reads", "elba_fe_B_dcsc", "elba_fe_get_B_dcsc", "elba_fe_device_B_dcsc",
     "elba_fe_contigs", "elba_fe_contigs_from_graph", "elba_fe_get_contig_layout", "elba_fe_get_contigs", "elba_fe_device_contigs",
+    "elba_fe_set_read_names", "elba_fe_paf", "elba_fe_get_paf", "elba_fe_device_paf",
 )
 
 _lib = None
@@ -311,11 +378,14 @@ class Context:
 
     ALIGN_FIELDS = ("begQ", "endQ", "begT", "endT", "score", "rc", "passed", "containedQ", "containedT", "direction", "directionT", "suffix", "suffixT")
 
-    def align(self, mat: int = 1, mis: int = -1, gap: int = -1, dropoff: int = 15):
+    def align(self, mat: int = 1, mis: int = -1, gap: int = -1, dropoff: int = 15, fetch: bool = True):
         """X-drop seed-and-extend of B's nonzeros (PairwiseAlignment, src/PairwiseAlignment.cpp:5-106; defaults src/main.cpp:53-56):
-        (rows, cols, fields[npairs, 13]) with global read ids, pairs in B's row-major order."""
+        (rows, cols, fields[npairs, 13]) with global read ids, pairs in B's row-major order.  fetch=False leaves the alignments
+        on the device and returns only their number."""
         n = C.c_uint64()
         self._ck(self.L.elba_fe_align(self.h, C.c_int(mat), C.c_int(mis), C.c_int(gap), C.c_int(dropoff), C.byref(n)))
+        if not fetch:
+            return int(n.value)
         rows, cols = np.zeros(n.value, np.int64), np.zeros(n.value, np.int64)
         out = np.zeros((n.value, len(self.ALIGN_FIELDS)), np.int32)
         self._ck(self.L.elba_fe_get_alignments(self.h, _p(rows), _p(cols), _p(out)))
@@ -386,6 +456,24 @@ class Context:
         self._ck(self.L.elba_fe_contigs_from_graph(self.h, _p(rows) if len(rows) else None, _p(cols) if len(rows) else None,
                                                    _p(fields) if len(rows) else None, C.c_uint64(len(rows)), C.byref(info)))
         return self._contigs_result(info)
+
+    def set_read_names(self, names):
+        """The names of the whole job's reads for the PAF text (elba_fe_set_read_names): names[r] is read r of the job (global id =
+        first id of rank 0 + r); str or bytes, checked by check_read_names.  An empty list clears them."""
+        b = check_read_names(names)
+        off = np.zeros(len(b) + 1, np.uint64)
+        off[1:] = np.cumsum([len(x) for x in b], dtype=np.uint64)
+        arena = np.frombuffer(b"".join(b), np.uint8) if b else np.zeros(0, np.uint8)
+        self._ck(self.L.elba_fe_set_read_names(self.h, _p(arena) if len(b) else None, _p(off) if len(b) else None, C.c_uint64(len(b))))
+
+    def paf(self, which: int = PAF_OVERLAP):
+        """PAF text formatted on the device (elba_fe_paf; the format is in include/elba_fe.h): (this rank's part as bytes, info
+        dict with lines, bytes, offset, total_lines, total_bytes, ms).  Collective on several GPUs."""
+        info = PafInfo()
+        self._ck(self.L.elba_fe_paf(self.h, C.c_int(which), C.byref(info)))
+        text = np.empty(max(info.bytes, 1), np.uint8)
+        self._ck(self.L.elba_fe_get_paf(self.h, _p(text)))
+        return text[:info.bytes].tobytes(), info.as_dict()
 
     def hll(self):
         regs, est = np.zeros(4096, np.uint8), C.c_double()

@@ -286,6 +286,42 @@ int elba_fe_get_contig_layout(elba_fe_ctx *ctx, uint64_t *ptr /* ncontigs + 1 */
 int elba_fe_get_contigs(elba_fe_ctx *ctx, uint8_t *packed, uint64_t *byte_off, uint64_t *len);
 int elba_fe_device_contigs(elba_fe_ctx *ctx, const uint8_t **packed, const uint64_t **byte_off, const uint64_t **len);
 
+/* ---- PAF text of the overlap graph and of the string graph (the reference's <prefix>.overlap.paf / .string.paf,
+ * src/main.cpp:303,317), formatted on the device.  The format (DESIGN.md §3d; restated in tests/paf_inputs.py; parity with the
+ * reference's own writer is UNPINNED): one line per alignment, 13 tab-separated columns, ending in '\n':
+ *     qname qlen begQ endQ strand tname tlen begT endT score max(endQ - begQ, endT - begT) 255 dr:i:<direction>
+ * q = the alignment's row read, t = its column read, strand '-' iff rc, the fields those of ELBA_FE_ALIGN_FIELDS (begT / endT
+ * are forward-strand coordinates of t); integers in plain decimal (int32 fields may be negative).  A read's name is the one
+ * elba_fe_set_read_names gave, else its global id in decimal.
+ * set_read_names: the names of the whole job's reads, job-relative: read r (global id = first id of rank 0 + r) is
+ *   names[name_off[r], name_off[r + 1]).  Checked on the host: every name non-empty, no byte <= 0x20 (ELBA_FE_ERR_INVALID).
+ *   The names stay until replaced; nreads == 0 clears them.  A count other than the job's reads makes elba_fe_paf
+ *   ELBA_FE_ERR_STATE.
+ * paf(ELBA_FE_PAF_OVERLAP): one line per alignment elba_fe_align made, passed or not (R before the prunes), in the order of
+ *   elba_fe_get_alignments; on several GPUs the ranks' parts follow in rank order (COLLECTIVE: one all-gather of the byte counts
+ *   gives offset and the totals; every rank formats its own alignments).  After elba_fe_align, else ELBA_FE_ERR_STATE.
+ * paf(ELBA_FE_PAF_STRING): one line per entry of the resident S with transposed == 0, in S's row-major order (each surviving
+ *   overlap once, in the orientation the aligner produced), printed from the entry's source alignment.  Needs the S that
+ *   elba_fe_reduce_overlap_graph left for the current R and the reads elba_fe_align saw (ELBA_FE_ERR_STATE otherwise).  Several
+ *   GPUs: COLLECTIVE (one sum all-reduce of 6 int32 per line); every rank formats the lines elba_fe_block_extent(lines, nranks,
+ *   rank).  The bytes of the whole file do not depend on the number of GPUs or the grid.
+ * info: this rank's part (lines, bytes, its byte offset in the whole file) and the whole file's totals; the rank parts laid
+ *   end to end at their offsets are the file.  get_paf copies this rank's part (info.bytes) to the host, device_paf hands out
+ *   the device pointer.  The text is that of the last elba_fe_paf; calls that discard the alignments, R or S, replace the reads
+ *   or set the names discard it (the getters are ELBA_FE_ERR_STATE until the next elba_fe_paf). */
+#define ELBA_FE_PAF_OVERLAP 0
+#define ELBA_FE_PAF_STRING  1
+typedef struct {
+    uint64_t lines, bytes;              /* this rank's part */
+    uint64_t offset;                    /* byte offset of this rank's part in the whole file */
+    uint64_t total_lines, total_bytes;  /* whole job */
+    float ms; float reserved;           /* device time of the call */
+} elba_fe_paf_info_t;
+int elba_fe_set_read_names(elba_fe_ctx *ctx, const char *names, const uint64_t *name_off /* nreads + 1 */, uint64_t nreads);
+int elba_fe_paf(elba_fe_ctx *ctx, int which, elba_fe_paf_info_t *info);
+int elba_fe_get_paf(elba_fe_ctx *ctx, char *text /* info.bytes */);
+int elba_fe_device_paf(elba_fe_ctx *ctx, const char **text);
+
 /* ---- the reference's sizing sketches, bit-exact (not needed for the result when lower >= 2) ----------- */
 /* HyperLogLog over the canonical k-mers of the uploaded reads exactly as KmerEstimateHandler drives it
  * (include/KmerOps.hpp:58-69, src/HyperLogLog.cpp:40-76): registers[4096] and estimate(). */
